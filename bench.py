@@ -1,6 +1,7 @@
 """bench.py — CADRE learner hot path on B200: encoder forward + GAE + PPO update (+ gradient all-reduce + Adam).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl cadre|reference] [--config cfg3|cfg5]
+                    [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...        (N > 1)
 
 One STEP = one learner iteration on every rank (weak scaling: per-GPU work is fixed):
@@ -33,6 +34,10 @@ import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True     # a benchmark run leaves the tree as build() left it (it may be read-only)
+
+DUMP_MAX_ELEMS = 1 << 22           # --dump-outputs: a larger output is written as a fixed, seeded sample of this size
+DUMP_MAX_BYTES = 64 << 20
 
 SEQ, MB_NUM, PPO_EPOCH = 8, 2, 4
 CONFIGS = {
@@ -161,6 +166,25 @@ def bind_to_gpu_numa_node(local_rank):
     except Exception:
         pass
     return None, None
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each array as <out_dir>/<name>.npy in float32. An array of more than DUMP_MAX_ELEMS elements is written as
+    the elements at DUMP_MAX_ELEMS flat positions drawn without replacement from a generator seeded with 0, in
+    ascending order: the same positions for the same shape, so that two runs or two builds compare element for
+    element."""
+    os.makedirs(out_dir, exist_ok=True)
+    total = 0
+    for name, t in arrays.items():
+        flat = t.detach().reshape(-1)
+        if flat.numel() > DUMP_MAX_ELEMS:
+            pos = np.sort(np.random.default_rng(0).choice(flat.numel(), DUMP_MAX_ELEMS, replace=False))
+            a = flat[torch.from_numpy(pos).to(flat.device)].float().cpu().numpy()
+        else:
+            a = t.detach().float().cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+        total += a.nbytes
+    assert total <= DUMP_MAX_BYTES, f"--dump-outputs wrote {total} bytes"
 
 
 # ---------------------------------------------------------------------------------------------- reference arm
@@ -396,6 +420,12 @@ def run_cadre(args):
         torch.cuda.profiler.stop()
         return
     ms_step, clocks = timed(step_resident, args.steps, args.warmup, sample=True)
+    if args.dump_outputs and rank == 0:
+        # what the last timed step handed its caller, before the e2e runs below go on updating the same learner
+        dump_outputs(args.dump_outputs, {"features": b["obs"], "returns": b["returns"], "advantages": b["advantages"],
+                                         "losses": learner.losses, "params": learner.params, "grads": learner.grads})
+    if args.dump_outputs and world > 1:
+        dist.barrier()      # the other ranks' next all-reduces must not wait on rank 0's dump
     ms_e2e, _ = timed(step_e2e, args.steps, max(3, args.warmup - 1))
     h2d_unique = ingest.h2d_bytes_last
     total_frames = FRAMES_PER_STEP * world
@@ -572,7 +602,8 @@ def run_cadre(args):
             # GPU-side bar (SURVEY.md §8d): the reference graph in torch eager (cuDNN / cuBLAS) on the same B200, in a
             # separate process so that no library kernel is ever loaded into the measured one
             try:
-                r = subprocess.run([sys.executable, os.path.join(ROOT, "tools", "gpu_eager_baseline.py"), "--json-line"],
+                r = subprocess.run([sys.executable, "-B", os.path.join(ROOT, "tools", "gpu_eager_baseline.py"),
+                                    "--json-line"],
                                    capture_output=True, text=True, timeout=600)
                 eager = json.loads(r.stdout.strip().splitlines()[-1])
                 eager["cadre_encoder_ms_b640"] = round(sum(k["ms"] for k in kernels) * 640.0 / nb, 3)
@@ -622,7 +653,16 @@ def main():
     ap.add_argument("--no-full-windows", action="store_true")
     ap.add_argument("--profile-step", action="store_true",
                     help="run ONE resident step inside cudaProfilerStart/Stop and exit (ncu --profile-from-start off)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last resident step computed on rank 0 to DIR/<name>.npy "
+                         "(float32): rollout features, returns, advantages, the raw losses [worker, head, (value loss, "
+                         "action loss, entropy)] of the last update step before the loss coefficients, parameters and "
+                         f"gradient; arrays of more than {DUMP_MAX_ELEMS} elements as a fixed, seeded sample")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.profile_step):
+        ap.error("--dump-outputs needs the timed steps of --impl cadre (not --impl reference or --profile-step)")
     args.warmup = max(args.warmup, 0)
     if args.impl == "reference":
         run_reference(args)

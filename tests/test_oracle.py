@@ -58,9 +58,15 @@ def test_encoder_matches_golden(golden_dir, tag, peaky):
     x = torch.from_numpy(R.pre_process(tick["rgb"], tick["route_fig"].copy()))
     with torch.no_grad():
         l4 = R.backbone(x, sd)
+        da = R.da_head(l4, sd)
         lat = R.encoder_latent(x, sd)
     assert np.array_equal(l4[:, :8].numpy(), g[f"{tag}_l4_slice"])
     assert np.array_equal(lat.numpy(), g[f"{tag}_latent"])
+    # (sum, L2 norm, max |x|) of the whole backbone output and of the attention head (PAM + CAM branches)
+    for t, key in ((l4, "l4_stats"), (da, "da_stats")):
+        t = t.double().flatten()
+        np.testing.assert_allclose([t.sum().item(), t.norm().item(), t.abs().max().item()], g[f"{tag}_{key}"],
+                                   rtol=1e-12, atol=0)
     # the peaky fixture must actually be far from a uniform softmax to stress the attention kernels
     if peaky:
         assert np.abs(g["peaky_latent"] - g["base_latent"]).max() > 1e-3
