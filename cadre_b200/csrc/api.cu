@@ -118,4 +118,31 @@ int cadre_conv2d_nhwc_bordered_out(const void* in, int B, int Hin, int Win, int 
   CADRE_API_END
 }
 
+int cadre_conv2d_nhwc_shortcut(const void* in, int B, int Hin, int Win, int Cin, const void* w, int Cout, int KH, int KW,
+                               int pad, const float* bias, int act, void* out, int in_pad, int out_pad, const void* in2,
+                               int Cin2, int Hin2, int Win2, int in2_pad, void* stream) {
+  CADRE_API_BEGIN
+  CADRE_REQUIRE(in2 != nullptr, "conv2d_nhwc_shortcut needs the shortcut input");
+  cadre::ConvArgs a;
+  a.in_pad = in_pad, a.out_pad = out_pad;
+  a.in = static_cast<const cadre::enc_t*>(in);
+  a.B = B, a.Hin = Hin, a.Win = Win, a.Cin = Cin;
+  a.w = static_cast<const cadre::enc_t*>(w);
+  a.Cout = Cout, a.KH = KH, a.KW = KW, a.stride = 1, a.pad = pad;
+  a.bias = bias, a.act = act, a.out = static_cast<cadre::enc_t*>(out);
+  a.in2 = static_cast<const cadre::enc_t*>(in2), a.Cin2 = Cin2, a.in2_pad = in2_pad, a.Hin2 = Hin2, a.Win2 = Win2;
+  cadre::launch_conv(a, static_cast<cudaStream_t>(stream));
+  CADRE_API_END
+}
+
+int cadre_stem_pool(const void* in, int B, const void* w, const float* bias, void* out, void* stream) {
+  CADRE_API_BEGIN
+  CADRE_REQUIRE(in && w && bias && out && B > 0, "stem_pool arguments");
+  cadre::StemArgs a;
+  a.in = static_cast<const cadre::enc_t*>(in), a.B = B;
+  a.w = static_cast<const cadre::enc_t*>(w), a.bias = bias, a.out = static_cast<cadre::enc_t*>(out);
+  cadre::launch_stem_pool(a, static_cast<cudaStream_t>(stream));
+  CADRE_API_END
+}
+
 }  // extern "C"

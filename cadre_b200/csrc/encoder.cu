@@ -382,6 +382,7 @@ int cadre_encoder_buffer(void* handle, int which, void** ptr, int64_t* elems_per
     case 3: *ptr = e->sa, *elems_per_frame = 40 * 128; break;          // PAM output
     case 4: *ptr = e->sc, *elems_per_frame = 40 * 128; break;          // CAM output
     case 5: *ptr = e->fc1, *elems_per_frame = 3072; break;             // six folded Linear(20480,512) + LeakyReLU
+    case 6: *ptr = e->padded, *elems_per_frame = 75 * 262 * 8; break;  // ingested image, stem input layout
     default: throw cadre::Error(1, "encoder_buffer: unknown buffer id");
   }
   CADRE_API_END

@@ -88,6 +88,20 @@ int cadre_conv3x3_flat128(const void* in, int B, int H, int W, const void* w, co
 int cadre_conv2d_nhwc_bordered_out(const void* in, int B, int Hin, int Win, int Cin, const void* w, int Cout, int KH,
                                    int KW, int stride, int pad, const float* bias, int act, void* out, int in_pad,
                                    void* stream);
+/* Stride-1 convolution with a fused ResNet shortcut (resnet.py:47-53, layer2.0 / 3.0 / 4.0 conv2 + downsample):
+ * out = act(conv(in, w[:, :KH*KW*Cin]) + conv1x1/s2(in2, w[:, KH*KW*Cin:]) + bias), the shortcut read on the
+ * stride-2 sub-lattice of in2 [B][Hin2 (+2)][Win2 (+2)][Cin2] as Cin2/64 extra k-blocks of one implicit GEMM.
+ * w is [Cout][KH*KW*Cin + Cin2] (the 1x1 weights appended along K), bias the sum of both biases;
+ * (Hin2 - 1) / 2 + 1 must equal the output height (likewise for the width). in_pad / in2_pad: the input is stored
+ * with a 1-pixel zero border; out_pad: out is [B][Hout+2][Wout+2][Cout] and its border is left untouched. */
+int cadre_conv2d_nhwc_shortcut(const void* in, int B, int Hin, int Win, int Cin, const void* w, int Cout, int KH, int KW,
+                               int pad, const float* bias, int act, void* out, int in_pad, int out_pad, const void* in2,
+                               int Cin2, int Hin2, int Win2, int in2_pad, void* stream);
+/* Fused stem (resnet.py:169-172): conv7x7/s2/p3 + folded BN bias -> ReLU -> MaxPool2d(3, 2, 1). in is the
+ * row-pair interleaved padded image [B][75][262][2][4] (padded row 2*y2 + r, image at rows / columns 3..146 / 3..258),
+ * w / bias as cadre_encoder_weights.stem_w / stem_b; out is the zero-bordered [B][38][66][64]: only its interior is
+ * written, the caller zeroes the border once. */
+int cadre_stem_pool(const void* in, int B, const void* w, const float* bias, void* out, void* stream);
 
 /* ------------------------------------------------------------------------------------------------------
  * Perception encoder forward = DANet.get_latent_feature(x, "concate")
@@ -125,7 +139,8 @@ int cadre_encoder_forward_u8(void* handle, const uint8_t* rgb, const uint8_t* ro
                              const double* measurements, int B, float* out, int ld_out, void* stream);
 /* x fp32 NCHW [B][4][144][256] already pre-processed (BASELINE config 2, encoder sweep). */
 int cadre_encoder_forward_f32(void* handle, const float* x_nchw, int B, float* out, int ld_out, void* stream);
-/* internal activation buffers for parity tests: 0 layer4 out, 1 feat_sum, 2 conv5a|5c, 3 PAM, 4 CAM, 5 stem */
+/* internal activation buffers for parity tests: 0 layer4 out, 1 feat_sum, 2 conv5a|5c, 3 PAM, 4 CAM, 5 fc1 (six folded
+ * Linear(20480,512) + LeakyReLU), 6 the ingested image [75][262][2][4] per frame (the input of cadre_stem_pool) */
 int cadre_encoder_buffer(void* handle, int which, void** ptr, int64_t* elems_per_frame);
 /* Re-runs the trunk on the frames ingested by the previous forward call with a CUDA event between launches:
  * ms_out[i] = device time of launch i (<= 64), names_out = ';'-joined launch names. Measurement helper for

@@ -279,13 +279,17 @@ def _conv_ops():
     return _lib, _lib.lib(), _lib.enc_dtype()
 
 
-@pytest.mark.parametrize("B,res", [(1, False), (3, True), (37, True), (640, False)])
-def test_halo128_conv_matches_fp32_conv_and_implicit_gemm_kernel(B, res):
-    """cadre_conv3x3_flat128 (BasicBlock conv of ResNet layer2, resnet.py:39-55: conv3x3 + folded BN bias (+ residual) +
-    ReLU on [B][20][34][128] bordered activations) against torch's fp32 convolution of the same fp16 operands and against
-    the implicit-GEMM kernel (cadre_conv2d_nhwc) it replaces; the zero border must come back exactly zero. B = 37 gives
-    an odd number of 128-pixel tiles (the last group's second tile is empty), B = 640 is the benchmarked chunk."""
+@pytest.mark.parametrize("B,res,act", [(1, False, 1), (3, True, 1), (37, True, 1), (640, False, 1), (3, True, 0),
+                                       (37, False, 0)])
+def test_halo128_conv_matches_fp32_conv_and_implicit_gemm_kernel(B, res, act):
+    """cadre_conv3x3_flat128 (BasicBlock conv of ResNet layer2, resnet.py:39-55: conv3x3 + folded BN bias (+ residual)
+    (+ ReLU) on [B][20][34][128] bordered activations) against the float64 convolution of the same fp16 operands,
+    element by element (the bound of test_encoder_kernels_gpu.py), and against the implicit-GEMM kernel
+    (cadre_conv2d_nhwc) it replaces; the zero border must come back exactly zero and nothing outside the output may
+    change. B = 37 gives an odd number of 128-pixel tiles (the last group's second tile is empty), B = 640 is the
+    benchmarked chunk."""
     import torch.nn.functional as F
+    from test_encoder_kernels_gpu import C_ACC, Guarded, _border_is, _check_bound
     _lib, L, dt = _conv_ops()
     H, W, C = 18, 32, 128
     g = torch.Generator(device="cuda").manual_seed(100 + B)
@@ -300,21 +304,26 @@ def test_halo128_conv_matches_fp32_conv_and_implicit_gemm_kernel(B, res):
         r = torch.randn(B, H, W, C, device="cuda", generator=g).to(dt)
         rp = torch.zeros_like(xp)
         rp[:, 1:-1, 1:-1] = r
-    out = torch.full((B, H + 2, W + 2, C), 7.0, device="cuda", dtype=dt)
-    _lib.check(L.cadre_conv3x3_flat128(_lib.ptr(xp), B, H, W, _lib.ptr(w_k), _lib.ptr(bias), _lib.ptr(rp), 1,
+    guarded = Guarded((B, H + 2, W + 2, C), 7.0, dtype=dt)
+    out = guarded.t
+    _lib.check(L.cadre_conv3x3_flat128(_lib.ptr(xp), B, H, W, _lib.ptr(w_k), _lib.ptr(bias), _lib.ptr(rp), act,
                                        _lib.ptr(out), _lib.stream_ptr()))
     old = torch.full((B, H, W, C), 7.0, device="cuda", dtype=dt)
-    _lib.check(L.cadre_conv2d_nhwc(_lib.ptr(xp), B, H, W, C, _lib.ptr(w_k), C, 3, 3, 1, 1, _lib.ptr(bias), _lib.ptr(r), 0, 1,
-                                   _lib.ptr(old), 1, _lib.stream_ptr()))
+    _lib.check(L.cadre_conv2d_nhwc(_lib.ptr(xp), B, H, W, C, _lib.ptr(w_k), C, 3, 3, 1, 1, _lib.ptr(bias), _lib.ptr(r), 0,
+                                   act, _lib.ptr(old), 1, _lib.stream_ptr()))
     torch.cuda.synchronize()
-    ref = F.conv2d(x.float(), w.float(), bias, stride=1, padding=1)
+    guarded.check()
+    ref = F.conv2d(x.double(), w.double(), bias.double(), stride=1, padding=1)
+    S = F.conv2d(x.double().abs(), w.double().abs(), bias.double().abs(), stride=1, padding=1)
     if res:
-        ref = ref + r.float().permute(0, 3, 1, 2)
-    ref = ref.relu().permute(0, 2, 3, 1)
+        ref = ref + r.double().permute(0, 3, 1, 2)
+        S = S + r.double().abs().permute(0, 3, 1, 2)
+    if act:
+        ref = ref.relu()
+    ref, S = ref.permute(0, 2, 3, 1), S.permute(0, 2, 3, 1)
     got = out[:, 1:-1, 1:-1].float()
-    border = out.float().clone()
-    border[:, 1:-1, 1:-1] = 0
-    assert float(border.abs().max()) == 0.0
+    assert _border_is(out, 0.0)
+    _check_bound("halo128", got, ref, S, C_ACC["halo128"])
     assert rel_l2(got, ref) < 1e-3                       # fp16 output rounding only (2^-11 relative per element)
     assert rel_l2(got, old.float()) < 1e-3
     assert float((got - ref).abs().max()) < 2e-2 * float(ref.abs().max())

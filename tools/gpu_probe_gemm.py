@@ -191,14 +191,14 @@ def run_stem(B, name="stem"):
     wk = torch.zeros(64, 8, 8, 4, device=dev, dtype=ENC16)   # [o][kh][kw][c]
     wk[:, :7, :7, :] = w.permute(0, 2, 3, 1)
     wk = wk.view(64, 4, 2, 8, 4).permute(0, 1, 3, 2, 4).contiguous().view(64, 256)
-    out = torch.full((B, 72, 128, 64), 7.0, device=dev, dtype=ENC16)
-    rc = L.cadre_stem_conv(_lib.ptr(xp), B, _lib.ptr(wk), _lib.ptr(bias), _lib.ptr(out), _lib.stream_ptr())
+    out = torch.zeros(B, 38, 66, 64, device=dev, dtype=ENC16)    # zero-bordered pooled map (interior written)
+    rc = L.cadre_stem_pool(_lib.ptr(xp), B, _lib.ptr(wk), _lib.ptr(bias), _lib.ptr(out), _lib.stream_ptr())
     if rc != 0:
         print(f"FAIL {name}: rc={rc} {L.cadre_last_error().decode()}", flush=True)
         return False
     torch.cuda.synchronize()
-    ref = F.conv2d(x.float(), w.float(), bias, stride=2, padding=3).relu()
-    return report(name, out.float().permute(0, 3, 1, 2), ref, 1e-2)
+    ref = F.max_pool2d(F.conv2d(x.float(), w.float(), bias, stride=2, padding=3).relu(), 3, 2, 1)
+    return report(name, out[:, 1:-1, 1:-1].float().permute(0, 3, 1, 2), ref, 1e-2)
 
 
 def timed(fn, iters=20):
