@@ -7,7 +7,11 @@ route normalisation, agent.py:43-75). So, per environment, seven of the eight [5
 already computed for the previous tick. `BatchedActor` keeps them in a device ring, encodes only the newest frame of
 each of E environments in one batch (E frames instead of 8E), and runs the per-command LSTM + actor-critic once for
 all E environments (rows routed by command). Results equal E independent `CadreAgent.act` calls on the full windows;
-only the order of the host-side Categorical draws differs (environment-major here)."""
+only the order of the host-side Categorical draws differs (environment-major here).
+
+`act_into` / `bootstrap_into` are the device-side rollout path: actions are drawn on the device by a counter-based
+sampler keyed by (seed, env id, tick) (include/cadre_b200.h, cadre_categorical_sample) and the whole tick is written
+into a RolloutPool by one kernel, so a tick costs the same number of launches and copies for any number of workers."""
 from types import SimpleNamespace
 
 import numpy as np
@@ -18,8 +22,10 @@ from . import ppo as _ppo
 
 
 class BatchedActor:
-    def __init__(self, agent, num_envs, verify_window=True):
-        """agent: a cadre_b200.agent.CadreAgent (owns the encoder and the flat PPO parameters)."""
+    def __init__(self, agent, num_envs, verify_window=True, seed=0, env_ids=None):
+        """agent: a cadre_b200.agent.CadreAgent (owns the encoder and the flat PPO parameters). `seed` and `env_ids`
+        (default 0..E-1) key the device-side sampler of `act_into`: environment e's draw at a tick depends only on
+        (seed, env_ids[e], tick, its log-probabilities), not on the batch it is stepped in."""
         self.agent, self.E = agent, int(num_envs)
         self.device = agent.device
         self.F, self.S = agent.lstm_input, 8
@@ -41,6 +47,17 @@ class BatchedActor:
         self._meas_h = torch.empty(self.E, 3, dtype=torch.float64, pin_memory=True)
         self._cmd_h = torch.empty(self.E, 1, dtype=torch.int32, pin_memory=True)
         self.frames_encoded = 0
+        # device-side rollout path (act_into / bootstrap_into)
+        self.seed = int(seed)
+        self.env_ids = list(range(self.E)) if env_ids is None else [int(i) for i in env_ids]
+        if len(self.env_ids) != self.E:
+            raise ValueError(f"env_ids has {len(self.env_ids)} entries for {self.E} environments")
+        self.ticks = 0                                       # act_into calls so far: the sampler's tick counter
+        self._env_ids_d = torch.tensor(self.env_ids, dtype=torch.int32, device=self.device)
+        self._rows = z(2, self.E, _ppo.ROW_OUT)
+        self._act_d = z(self.E, 2, dtype=torch.int64)
+        self._act_h = torch.empty(self.E, 2, dtype=torch.int64, pin_memory=True)
+        self._boot = None
 
     # ------------------------------------------------------------------ perception with the frame cache
     def _slid_by_one(self, e, tick):
@@ -99,11 +116,7 @@ class BatchedActor:
         values [E,2]) on the device; column 0 = steer, 1 = throttle. One Categorical draw per head for the whole
         batch (distributions.py:96-99 semantics, environment-major draw order)."""
         feats = self.encode(ticks)
-        for e, t in enumerate(ticks):
-            self._cmd_h[e, 0] = int(t["command"])
-        cmd = self._cmd_h.to(self.device, non_blocking=True)
-        for st in self._st:
-            st.command.copy_(cmd)
+        self._upload_commands(ticks)
         out = self._engine.evaluate([tuple(self._st)], [self._adv], self._idx, self.agent.owner.params)  # [2, E, 36]
         actions, log_probs = [], []
         for h, A in ((0, 33), (1, 3)):
@@ -112,6 +125,58 @@ class BatchedActor:
             actions.append(a)
             log_probs.append(logits.gather(1, a))
         return feats, torch.cat(actions, 1), torch.cat(log_probs, 1), out[:, :, 0].t().contiguous()
+
+    def _upload_commands(self, ticks):
+        for e, t in enumerate(ticks):
+            self._cmd_h[e, 0] = int(t["command"])
+        cmd = self._cmd_h.to(self.device, non_blocking=True)
+        for st in self._st:
+            st.command.copy_(cmd)
+
+    def act_into(self, ticks, pool):
+        """One tick of all E environments written straight into `pool` (a RolloutPool with E workers) at its cursor:
+        encoder batch, PPO forward, then one kernel that draws both heads' actions on the device and stores obs,
+        action, log-prob, value, command and (below slot num_steps) hn / cn of all 2E storages; one device-to-host
+        copy of the actions. Every storage's cursor advances like `RolloutStorage.insert`'s (modulo num_steps + 1).
+        Rewards and masks follow with `pool.write_env_results`. Returns the actions, int64 [E, 2] (host)."""
+        if pool.workers != self.E:
+            raise ValueError(f"pool has {pool.workers} workers, the actor steps {self.E} environments")
+        slot = pool.storages[0][0].step
+        self.encode(ticks)
+        self._upload_commands(ticks)
+        self._engine.act([tuple(self._st)], [self._adv], self._idx, self.agent.owner.params, self._rows, pool.c_ref(),
+                         slot, self.seed, self.ticks, self._env_ids_d, self.agent.hidden_state, self._act_d)
+        self._act_h.copy_(self._act_d, non_blocking=True)
+        torch.cuda.current_stream(self.device).synchronize()
+        self.ticks += 1
+        for pair in pool.storages:
+            for st in pair:
+                st.step = (st.step + 1) % (st.num_steps + 1)
+        return self._act_h.numpy().copy()
+
+    def bootstrap_into(self, pool, done):
+        """pool.next_value [2W] = the bootstrap values of agent.get_value (train.py:76-79) for all W workers in one
+        forward: each storage's obs[T] / command[T] (get_last reads slot T whatever the cursor is) and the agent's
+        hidden_state; exactly 0 for a worker whose last tick was `done`. No host synchronisation."""
+        W, T = pool.workers, pool.num_steps
+        if len(done) != W:
+            raise ValueError(f"done has {len(done)} entries for {W} workers")
+        if self._boot is None or self._boot[0] is not pool:
+            z = lambda *s: torch.zeros(*s, device=self.device)  # noqa: E731
+            eng = _ppo.PpoEngine(W, 1, self.agent.clip, self.agent.value_coeff, self.agent.clip_coeff,
+                                 self.agent.ent_coeff, self.device)
+            hid = z(2, T + 1, self.F)                  # row T: the agent's hidden_state, read through index T
+            zero = z(T + 1, 1)                         # advantages slot: read by the gather, unused by the forward
+            sts = [tuple(SimpleNamespace(obs=st.obs, action=st.action, value_preds=st.value_preds, returns=st.returns,
+                                         action_log_probs=st.action_log_probs, hn=hid[0], cn=hid[1], command=st.command)
+                         for st in pair) for pair in pool.storages]
+            self._boot = (pool, eng, hid, sts, [(zero, zero)] * W, [[[T], [T]] for _ in range(W)], z(2, W, _ppo.ROW_OUT))
+        _, eng, hid, sts, advs, idx, rows = self._boot
+        hid[0, T].copy_(self.agent.hidden_state[0].reshape(-1))
+        hid[1, T].copy_(self.agent.hidden_state[1].reshape(-1))
+        mask = sum(1 << w for w in range(W) if done[w])
+        eng.bootstrap(sts, advs, idx, self.agent.owner.params, rows, mask, pool.next_value)
+        return pool.next_value
 
     def act(self, ticks):
         """Reference-shaped results: per environment the 5-tuple of CadreAgent.act: (feature [8,530],

@@ -20,6 +20,7 @@
 #include "ptx.cuh"
 #include "ppo_layout.h"
 #include "lstm_seq.cuh"
+#include "sampler.cuh"
 
 #include <algorithm>
 #include <cmath>
@@ -535,6 +536,63 @@ __global__ void __launch_bounds__(256) head_eval_kernel(const float* __restrict_
   if (lane == 0) o[0] = v, o[1] = lp, o[2] = ent;
   if (lane < A) o[3 + lane] = lp0;            // normalised logits (Categorical.logits)
   if (lane + 32 < A) o[3 + lane + 32] = lp1;
+}
+
+// Act step tail (cadre_ppo_act): block e samples both heads of environment e from head_eval_kernel's rows
+// (row_out[(head * E + e) * ROW_OUT], W = 1) and writes the tick of storages 2e, 2e + 1 into the pool at `slot`
+// (storage.py:45-58: everything but rewards / masks, which come from env.step afterwards).
+__global__ void __launch_bounds__(256) act_write_kernel(const float* __restrict__ row_out, int E_env,
+                                                        cadre_rollout_pool pool, int slot, unsigned long long seed,
+                                                        unsigned long long tick, const int* __restrict__ env_ids,
+                                                        const float* __restrict__ window,
+                                                        const int* __restrict__ command,
+                                                        const float* __restrict__ hid_h,
+                                                        const float* __restrict__ hid_c,
+                                                        long long* __restrict__ actions_out) {
+  pdl_trigger();
+  pdl_wait();
+  const int e = blockIdx.x;
+  const long long T1 = pool.num_steps + 1;
+  if (threadIdx.x < 2) {
+    const int h = threadIdx.x, A = h == 0 ? 33 : 3;
+    const float* row = row_out + (static_cast<long long>(h) * E_env + e) * ROW_OUT;
+    const float u = philox_uniform(philox_word(philox_words(seed, tick, env_ids[e]), h));
+    const int a = categorical_draw(row + 3, A, u);
+    const long long at = (2LL * e + h) * T1 + slot;
+    pool.action[at] = a;
+    pool.action_log_probs[at] = row[3 + a];
+    pool.value_preds[at] = row[0];
+    pool.command[at] = command[e];
+    actions_out[2 * e + h] = a;
+  }
+  const int win = pool.seq_length * pool.feature_dims;
+  const float* src = window + static_cast<long long>(e) * win;
+  float* d0 = pool.obs + (2LL * e * T1 + slot) * win;
+  float* d1 = d0 + T1 * win;
+  for (int k = threadIdx.x; k < win; k += blockDim.x) {
+    const float v = src[k];
+    d0[k] = v, d1[k] = v;
+  }
+  if (slot < pool.num_steps) {   // storage.py:84-87
+    const int H = pool.hidden_size;
+    const long long o0 = (2LL * e * T1 + slot + 1) * H, o1 = o0 + T1 * H;
+    for (int k = threadIdx.x; k < H; k += blockDim.x) {
+      const float vh = hid_h[k], vc = hid_c[k];
+      pool.hn[o0 + k] = vh, pool.hn[o1 + k] = vh;
+      pool.cn[o0 + k] = vc, pool.cn[o1 + k] = vc;
+    }
+  }
+}
+
+// Bootstrap tail (cadre_ppo_bootstrap, mini_batch = 1): next_value[w][h] = value of row (h, w), 0 for a done worker.
+__global__ void bootstrap_value_kernel(const float* __restrict__ row_out, int W, unsigned long long done_mask,
+                                       float* __restrict__ next_value) {
+  pdl_trigger();
+  pdl_wait();
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= 2 * W) return;
+  const int w = i >> 1, h = i & 1;
+  next_value[i] = ((done_mask >> w) & 1ull) ? 0.f : row_out[(static_cast<long long>(h) * W + w) * ROW_OUT];
 }
 
 // column sums over the valid rows of each expert (bias gradients); deterministic
@@ -1083,6 +1141,57 @@ int cadre_ppo_evaluate(void* handle, const cadre_storage_ref* storages_host, con
                                                              P->sc.action, P->R, P->cap, row_out);
   CADRE_CUDA_CHECK(cudaGetLastError());
   P->launches = n + 1;
+  CADRE_API_END
+}
+
+int cadre_ppo_act(void* handle, const cadre_storage_ref* storages_host, const int32_t* indices_host,
+                  const float* params, float* row_out, const cadre_rollout_pool* pool, int slot, uint64_t seed,
+                  uint64_t tick, const int32_t* env_ids, const float* hidden_hn, const float* hidden_cn,
+                  int64_t* actions_out, void* stream) {
+  CADRE_API_BEGIN
+  cadre::check_rollout_pool(pool, slot);
+  PpoPlan* P = static_cast<PpoPlan*>(handle);
+  CADRE_REQUIRE(P != nullptr, "ppo_act: ppo handle is NULL");
+  CADRE_REQUIRE(storages_host && indices_host && params && row_out && env_ids && hidden_hn && hidden_cn && actions_out,
+                "ppo_act pointers");
+  CADRE_REQUIRE(pool->obs && pool->action && pool->action_log_probs && pool->value_preds && pool->command && pool->hn &&
+                    pool->cn, "ppo_act: rollout pool pointers");
+  const int E_env = P->cfg.mini_batch;
+  CADRE_REQUIRE(P->cfg.workers == 1, "ppo_act needs an engine with workers = 1, mini_batch = E");
+  CADRE_REQUIRE(pool->storages == 2 * E_env, "ppo_act: the pool must hold 2 storages per environment");
+  CADRE_REQUIRE(pool->seq_length == 8 && pool->feature_dims == cadre::ppo::F && pool->hidden_size == cadre::ppo::F,
+                "ppo_act: pool windows must be [8][530] with hidden size 530");
+  for (int h = 0; h < 2; ++h)
+    for (int i = 0; i < E_env; ++i)
+      CADRE_REQUIRE(indices_host[h * E_env + i] == i, "ppo_act: indices must be 0..E-1 for both heads");
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  int n = cadre::ppo_forward(P, storages_host, indices_host, params, s);
+  cadre::launch_k(cadre::head_eval_kernel, dim3((2 * P->R + 7) / 8), dim3(256), 0, s, P->Y2, params, P->row_slot,
+                  P->row_expert, P->sc.action, P->R, P->cap, row_out);
+  cadre::launch_k(cadre::act_write_kernel, dim3(E_env), dim3(256), 0, s, row_out, E_env, *pool, slot,
+                  static_cast<unsigned long long>(seed), static_cast<unsigned long long>(tick), env_ids,
+                  storages_host[0].obs, storages_host[0].command, hidden_hn, hidden_cn,
+                  reinterpret_cast<long long*>(actions_out));
+  CADRE_CUDA_CHECK(cudaGetLastError());
+  P->launches = n + 2;
+  CADRE_API_END
+}
+
+int cadre_ppo_bootstrap(void* handle, const cadre_storage_ref* storages_host, const int32_t* indices_host,
+                        const float* params, float* row_out, uint64_t done_mask, float* next_value, void* stream) {
+  CADRE_API_BEGIN
+  PpoPlan* P = static_cast<PpoPlan*>(handle);
+  CADRE_REQUIRE(P != nullptr, "ppo_bootstrap: ppo handle is NULL");
+  CADRE_REQUIRE(storages_host && indices_host && params && row_out && next_value, "ppo_bootstrap pointers");
+  CADRE_REQUIRE(P->cfg.mini_batch == 1, "ppo_bootstrap needs an engine with mini_batch = 1");
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  int n = cadre::ppo_forward(P, storages_host, indices_host, params, s);
+  cadre::launch_k(cadre::head_eval_kernel, dim3((2 * P->R + 7) / 8), dim3(256), 0, s, P->Y2, params, P->row_slot,
+                  P->row_expert, P->sc.action, P->R, P->cap, row_out);
+  cadre::launch_k(cadre::bootstrap_value_kernel, dim3((2 * P->R + 127) / 128), dim3(128), 0, s, row_out, P->R,
+                  static_cast<unsigned long long>(done_mask), next_value);
+  CADRE_CUDA_CHECK(cudaGetLastError());
+  P->launches = n + 2;
   CADRE_API_END
 }
 

@@ -3,8 +3,27 @@
 #include "../../include/cadre_b200.h"
 #include "internal.h"
 #include "ptx.cuh"
+#include "sampler.cuh"
 
 namespace cadre {
+
+// Standalone form of the act step's sampler (sampler.cuh): one thread per row.
+__global__ void __launch_bounds__(128) categorical_sample_kernel(const float* __restrict__ logp, long long ld, int rows,
+                                                                 int A, unsigned long long seed, unsigned long long tick,
+                                                                 const int* __restrict__ env_ids, int word,
+                                                                 long long* __restrict__ action_out,
+                                                                 float* __restrict__ logp_out, float* __restrict__ u_out) {
+  pdl_trigger();
+  pdl_wait();
+  const int r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= rows) return;
+  const float u = philox_uniform(philox_word(philox_words(seed, tick, env_ids[r]), word));
+  const float* lp = logp + r * ld;
+  const int a = categorical_draw(lp, A, u);
+  action_out[r] = a;
+  logp_out[r] = lp[a];
+  if (u_out) u_out[r] = u;
+}
 
 // ---------------------------------------------------------------------------------------------------------
 // RolloutStorage.compute_returns (ppo_agent/storage.py:68-76, GAE branch) + advantage normalisation
@@ -386,6 +405,38 @@ int cadre_window_scatter(const float* unique_feats, float* obs, int workers, int
                   static_cast<cudaStream_t>(stream), unique_feats, obs, workers, num_steps, seq_length, feature_dims,
                   static_cast<long long>(obs_head_stride), static_cast<long long>(obs_step_stride));
   CADRE_CUDA_CHECK(cudaGetLastError());
+  CADRE_API_END
+}
+
+int cadre_categorical_sample(const float* logp, int ld, int rows, int A, uint64_t seed, uint64_t tick,
+                             const int32_t* env_ids, int word, int64_t* action_out, float* logp_out, float* u_out,
+                             void* stream) {
+  CADRE_API_BEGIN
+  CADRE_REQUIRE(A >= 1 && A <= 33, "categorical_sample: A must lie in [1, 33]");
+  CADRE_REQUIRE(rows > 0, "categorical_sample: rows must be positive");
+  CADRE_REQUIRE(ld >= A, "categorical_sample: ld must be at least A");
+  CADRE_REQUIRE(word >= 0 && word <= 3, "categorical_sample: word must lie in [0, 3]");
+  CADRE_REQUIRE(logp && env_ids && action_out && logp_out, "categorical_sample pointers");
+  cadre::launch_k(cadre::categorical_sample_kernel, dim3((rows + 127) / 128), dim3(128), 0,
+                  static_cast<cudaStream_t>(stream), logp, static_cast<long long>(ld), rows, A,
+                  static_cast<unsigned long long>(seed), static_cast<unsigned long long>(tick), env_ids, word,
+                  reinterpret_cast<long long*>(action_out), logp_out, u_out);
+  CADRE_CUDA_CHECK(cudaGetLastError());
+  CADRE_API_END
+}
+
+int cadre_rollout_env_results(const cadre_rollout_pool* pool, int slot, const float* rewards_host,
+                              const float* masks_host, void* stream) {
+  CADRE_API_BEGIN
+  cadre::check_rollout_pool(pool, slot);
+  CADRE_REQUIRE(pool->rewards && pool->masks && rewards_host && masks_host, "rollout_env_results pointers");
+  // one element per storage into the column [n][slot]: destination pitch = one storage's T + 1 floats
+  const size_t pitch = sizeof(float) * (static_cast<size_t>(pool->num_steps) + 1);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  CADRE_CUDA_CHECK(cudaMemcpy2DAsync(pool->rewards + slot, pitch, rewards_host, sizeof(float), sizeof(float),
+                                     pool->storages, cudaMemcpyHostToDevice, s));
+  CADRE_CUDA_CHECK(cudaMemcpy2DAsync(pool->masks + slot, pitch, masks_host, sizeof(float), sizeof(float),
+                                     pool->storages, cudaMemcpyHostToDevice, s));
   CADRE_API_END
 }
 

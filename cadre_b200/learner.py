@@ -11,11 +11,13 @@ replicas hold identical parameters afterwards. How it is done here:
   * every rank then runs the same deterministic clip + Adam kernel, so no parameter broadcast
     (agent.py:239-243) is needed and replicas stay bit-identical.
 """
+import ctypes
 import os
 
 import numpy as np
 import torch
 
+from . import _lib
 from . import ppo as _ppo
 from ._lib import CadreError
 from . import ppo_params
@@ -49,6 +51,38 @@ class RolloutPool:
                 pair.append(st)
             self.storages.append(tuple(pair))
         self.num_steps, self.gamma, self.tau = T, cfg["gamma"], cfg["tau"]
+        self._ref = None
+        self._env_h = None
+
+    def c_ref(self):
+        """The pool's batched tensors as a `cadre_rollout_pool` (ppo.RolloutPoolC) for the device-side rollout path."""
+        if self._ref is None:
+            b = self.batched
+            r = _ppo.RolloutPoolC()
+            for name in ("obs", "action", "action_log_probs", "value_preds", "rewards", "masks", "command", "hn", "cn"):
+                setattr(r, name, b[name].data_ptr())
+            r.storages, r.num_steps = self.workers * 2, self.num_steps
+            r.seq_length, r.feature_dims, r.hidden_size = b["obs"].shape[2], b["obs"].shape[3], b["hn"].shape[2]
+            self._ref = r
+        return self._ref
+
+    def write_env_results(self, slot, rewards, masks):
+        """Rewards and masks [W, 2] of every storage's slot `slot` (what `insert` stores from env.step, storage.py:45-58)
+        with two host-to-device copies, whatever W is. They are staged in pinned memory. In the rollout loop the host
+        rewrites that memory only after the next tick's action copy has synchronised the stream, so these copies are
+        done by then and the event wait below returns at once; it guards callers that skip the act step."""
+        if self._env_h is None:
+            self._env_h = torch.empty(2, self.workers * 2, dtype=torch.float32, pin_memory=True)
+            self._env_ev = torch.cuda.Event()
+        self._env_ev.synchronize()
+        h = self._env_h.numpy()
+        h[0] = np.asarray(rewards, dtype=np.float32).reshape(-1)
+        h[1] = np.asarray(masks, dtype=np.float32).reshape(-1)
+        with torch.cuda.device(self.device):
+            _lib.check(_lib.lib().cadre_rollout_env_results(
+                ctypes.byref(self.c_ref()), int(slot), ctypes.c_void_p(self._env_h.data_ptr()),
+                ctypes.c_void_p(self._env_h.data_ptr() + 4 * self.workers * 2), _lib.stream_ptr(self.device)))
+            self._env_ev.record()
 
     def compute_returns(self, next_values=None, normalize=True):
         """All 2W sequences in one launch (storage.py:68-76 + train.py:82-88). next_values: [W,2] or None to use

@@ -22,6 +22,13 @@ class StorageRefC(ctypes.Structure):
                                                "hn", "cn", "command")]
 
 
+class RolloutPoolC(ctypes.Structure):
+    """Mirror of `cadre_rollout_pool`: the batched device tensors of a RolloutPool (storage n = 2 * worker + head)."""
+    _fields_ = [(n, ctypes.c_void_p) for n in ("obs", "action", "action_log_probs", "value_preds", "rewards", "masks",
+                                               "command", "hn", "cn")] + \
+               [(n, ctypes.c_int32) for n in ("storages", "num_steps", "seq_length", "feature_dims", "hidden_size")]
+
+
 ROW_OUT = 36
 
 
@@ -125,6 +132,29 @@ class PpoEngine:
                                                     _lib.ptr(params), _lib.ptr(out), _lib.stream_ptr(self.device)))
         return out
 
+    def act(self, storages, advantages, indices, params, row_out, pool_ref, slot, seed, tick, env_ids, hidden, actions):
+        """cadre_ppo_act (workers = 1, mini_batch = E): `evaluate` into row_out [2, E, 36], then one kernel that draws
+        both heads' actions of every environment (env_ids int32 [E] on the device, counter-based sampler keyed by
+        seed / tick) and writes the tick into the pool `pool_ref` (RolloutPoolC) at `slot`; actions int64 [E, 2]."""
+        idx = self._marshal(storages, advantages, indices)
+        hn, cn = hidden
+        with torch.cuda.device(self.device):
+            _lib.check(self._lib.cadre_ppo_act(
+                self._h, self._refs, idx.ctypes.data_as(ctypes.c_void_p), _lib.ptr(params), _lib.ptr(row_out),
+                ctypes.byref(pool_ref), int(slot), ctypes.c_uint64(seed), ctypes.c_uint64(tick), _lib.ptr(env_ids),
+                _lib.ptr(hn), _lib.ptr(cn), _lib.ptr(actions), _lib.stream_ptr(self.device)))
+        return actions
+
+    def bootstrap(self, storages, advantages, indices, params, row_out, done_mask, next_value):
+        """cadre_ppo_bootstrap (mini_batch = 1): next_value [W, 2] = the value of each worker's row, 0 where bit w of
+        done_mask is set; no host synchronisation."""
+        idx = self._marshal(storages, advantages, indices)
+        with torch.cuda.device(self.device):
+            _lib.check(self._lib.cadre_ppo_bootstrap(
+                self._h, self._refs, idx.ctypes.data_as(ctypes.c_void_p), _lib.ptr(params), _lib.ptr(row_out),
+                ctypes.c_uint64(done_mask), _lib.ptr(next_value), _lib.stream_ptr(self.device)))
+        return next_value
+
     def adam_step(self, params, grads, exp_avg, exp_avg_sq, step, max_grad_norm=250.0, lr=3e-4, betas=(0.9, 0.999),
                   eps=1e-8):
         with torch.cuda.device(self.device):
@@ -178,6 +208,22 @@ class PpoEngine:
     @property
     def launches(self):
         return int(self._lib.cadre_ppo_launches(self._h))
+
+
+def categorical_sample(logp, A, seed, tick, env_ids, word, u_out=None):
+    """cadre_categorical_sample (include/cadre_b200.h): one draw per row of log-probabilities logp fp32 [rows, ld]
+    (columns >= A are never read) for environments env_ids int32 [rows]. Returns (action int64 [rows], logp fp32
+    [rows]); u_out (fp32 [rows] or None) receives the uniform of each draw."""
+    rows, ld = logp.shape
+    _check_tensor(logp, torch.float32, "logp")
+    _check_tensor(env_ids, torch.int32, "env_ids")
+    action = torch.empty(rows, dtype=torch.int64, device=logp.device)
+    lp = torch.empty(rows, dtype=torch.float32, device=logp.device)
+    with torch.cuda.device(logp.device):
+        _lib.check(_lib.lib().cadre_categorical_sample(
+            _lib.ptr(logp), int(ld), int(rows), int(A), ctypes.c_uint64(seed), ctypes.c_uint64(tick), _lib.ptr(env_ids),
+            int(word), _lib.ptr(action), _lib.ptr(lp), _lib.ptr(u_out), _lib.stream_ptr(logp.device)))
+    return action, lp
 
 
 def gae(rewards, values, masks, next_value, returns, adv, gamma=0.99, tau=0.95, normalize=True):

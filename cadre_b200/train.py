@@ -16,10 +16,17 @@ from .synthetic_env import SyntheticEnv
 
 
 def train(rank, train_cfg, agent_cfg, env_cfg, rollout_cfg, danet_state, ppo_state=None, workers=1, max_episode=None,
-          process_group=None, log=print, batched_acting=True):
+          process_group=None, log=print, batched_acting=True, device_rollout=False):
     """One rank: `workers` logical workers (env + rollout pair each) sharing one agent replica. With
     `batched_acting` the rank's workers are stepped together through `BatchedActor` (one encoder batch of the newest
-    frames + one routed LSTM / head evaluation per tick) instead of one `agent.act` call per worker."""
+    frames + one routed LSTM / head evaluation per tick) instead of one `agent.act` call per worker.
+    `device_rollout` (needs `batched_acting`) draws the actions on the device and writes each tick into the rollout
+    pool with a fixed number of launches and copies (`BatchedActor.act_into`, `RolloutPool.write_env_results`), and
+    bootstraps all workers' values in one forward (`BatchedActor.bootstrap_into`). Its draws come from a counter-based
+    generator keyed by (env seed, worker id, tick), not from torch's RNG, so its trajectories differ from the default
+    path's."""
+    if device_rollout and not batched_acting:
+        raise ValueError("device_rollout=True needs batched_acting=True")
     device = torch.device("cuda:" + str(agent_cfg.model_cfg.device_num))
     envs = [SyntheticEnv(dict(env_cfg, rank=rank * workers + w, seq_length=rollout_cfg.seq_length))
             for w in range(workers)]
@@ -36,25 +43,34 @@ def train(rank, train_cfg, agent_cfg, env_cfg, rollout_cfg, danet_state, ppo_sta
     obs = [e.reset() for e in envs]
     done = [False] * workers
     history = []
-    actor = BatchedActor(agent, workers) if batched_acting else None
+    if device_rollout:   # the same env ids as the SyntheticEnvs: a rollout split over ranks draws what one rank would
+        actor = BatchedActor(agent, workers, seed=env_cfg.get("seed", 0),
+                             env_ids=[rank * workers + w for w in range(workers)])
+    else:
+        actor = BatchedActor(agent, workers) if batched_acting else None
     for episode in range(max_episode if max_episode is not None else train_cfg.max_episode):
-        for _ in range(num_steps):                                        # train.py:55-74
-            acted = actor.act(obs) if actor is not None else None
-            for w, env in enumerate(envs):
-                command = obs[w]["command"]
-                feat, action, logp, value, hidden = acted[w] if acted is not None else agent.act(obs[w])
-                obs[w], reward, done[w], info = env.step(agent.convert_action(action))
-                for h in range(2):
-                    mask = torch.tensor([[0.0] if info["action_done"][h] else [1.0]])
-                    pool.storages[w][h].insert(feat, action[h], logp[h], value[h], reward[h], mask, hidden, command)
-                if done[w]:
-                    obs[w] = env.reset()
-                    if actor is not None:
-                        actor.reset(w)
-        nv = torch.zeros(workers, 2)
-        for w in range(workers):                                          # train.py:76-79
-            vs, vt = agent.get_value(done[w], pool.storages[w][0].get_last(), pool.storages[w][1].get_last())
-            nv[w, 0], nv[w, 1] = float(vs.reshape(-1)[0]), float(vt.reshape(-1)[0])
+        if device_rollout:
+            _device_rollout(actor, agent, envs, pool, obs, done, num_steps)
+            actor.bootstrap_into(pool, done)                              # train.py:76-79, into pool.next_value
+            nv = None
+        else:
+            for _ in range(num_steps):                                    # train.py:55-74
+                acted = actor.act(obs) if actor is not None else None
+                for w, env in enumerate(envs):
+                    command = obs[w]["command"]
+                    feat, action, logp, value, hidden = acted[w] if acted is not None else agent.act(obs[w])
+                    obs[w], reward, done[w], info = env.step(agent.convert_action(action))
+                    for h in range(2):
+                        mask = torch.tensor([[0.0] if info["action_done"][h] else [1.0]])
+                        pool.storages[w][h].insert(feat, action[h], logp[h], value[h], reward[h], mask, hidden, command)
+                    if done[w]:
+                        obs[w] = env.reset()
+                        if actor is not None:
+                            actor.reset(w)
+            nv = torch.zeros(workers, 2)
+            for w in range(workers):                                      # train.py:76-79
+                vs, vt = agent.get_value(done[w], pool.storages[w][0].get_last(), pool.storages[w][1].get_last())
+                nv[w, 0], nv[w, 1] = float(vs.reshape(-1)[0]), float(vt.reshape(-1)[0])
         pool.compute_returns(nv, normalize=train_cfg.use_adv_norm)        # train.py:81-88
         learner.learn(pool, train_cfg.ppo_epoch)                          # train.py:93-110
         L = learner.scaled_losses(mean=True).mean(0)     # mean over update steps and workers
@@ -62,6 +78,24 @@ def train(rank, train_cfg, agent_cfg, env_cfg, rollout_cfg, danet_state, ppo_sta
         if episode % train_cfg.log_interval == 0 and rank == 0:
             log("Episode: {}, value loss: {:.4f}, policy loss: {:.4f}, entropy loss: {:.4f}".format(episode, *L))
     return learner, history
+
+
+def _device_rollout(actor, agent, envs, pool, obs, done, num_steps):
+    """num_steps ticks of train.py:55-74 through the device path: act_into -> env.step x W -> write_env_results."""
+    W = len(envs)
+    rewards = np.zeros((W, 2), dtype=np.float32)
+    masks = np.zeros((W, 2), dtype=np.float32)
+    for _ in range(num_steps):
+        slot = pool.storages[0][0].step
+        actions = actor.act_into(obs, pool)
+        for w, env in enumerate(envs):
+            obs[w], reward, done[w], info = env.step(agent.convert_action(actions[w]))
+            rewards[w] = reward
+            masks[w] = [0.0 if d else 1.0 for d in info["action_done"]]
+            if done[w]:
+                obs[w] = env.reset()
+                actor.reset(w)
+        pool.write_env_results(slot, rewards, masks)
 
 
 def main():

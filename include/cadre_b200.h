@@ -242,6 +242,66 @@ int cadre_ppo_check(void* handle);
 int cadre_ppo_launches(void* handle);
 
 /* ------------------------------------------------------------------------------------------------------
+ * Device-side rollout collection: replaces the host-side Categorical draw (ppo_agent/distributions.py:96-99,
+ * agent.py:114-141), the per-worker RolloutStorage.insert calls (storage.py:45-58) and the per-worker get_value
+ * bootstrap (train.py:66-79) with a fixed number of launches and copies per tick, whatever the worker count.
+ *
+ * Counter-based categorical sampler (cadre_b200/csrc/sampler.cuh). A draw is a pure function of
+ * (seed, env id, tick, word, log-probs); the library holds no RNG state:
+ *   x = Philox4x32-10(counter = (tick & 0xffffffff, tick >> 32, env_id, 0), key = (seed & 0xffffffff, seed >> 32)),
+ *       output word `word` (the act step uses word 0 for the steer head, 1 for the throttle head);
+ *   u = (x >> 8) * 2^-24, exact in fp32;
+ *   p_j = expf(lp_j) for j < A (columns >= A are never read), c_j = inclusive prefix sum in index order;
+ *   a = min{ j : c_j > u * c_{A-1} }, or max{ j : p_j > 0 } if rounding leaves none; so p_j == 0 is never drawn.
+ * cadre_categorical_sample: rows of fp32 log-probabilities logp[rows][ld], env_ids int32 [rows] (device);
+ * action_out int64 [rows], logp_out fp32 [rows] = lp_a bit for bit, u_out fp32 [rows] = u (may be NULL).
+ * 1 <= A <= 33 (33 = steer, 3 = throttle), rows > 0, 0 <= word <= 3. */
+int cadre_categorical_sample(const float* logp, int ld, int rows, int A, uint64_t seed, uint64_t tick,
+                             const int32_t* env_ids, int word, int64_t* action_out, float* logp_out, float* u_out,
+                             void* stream);
+
+/* The batched tensors of a RolloutPool (cadre_b200/learner.py): `storages` = 2 * workers RolloutStorage objects,
+ * storage n = 2 * worker + head, each tensor [storages][num_steps + 1][...] contiguous (storage.py:8-26). */
+typedef struct cadre_rollout_pool {
+  float* obs;              /* [n][T+1][seq_length][feature_dims] */
+  int64_t* action;         /* [n][T+1] */
+  float* action_log_probs; /* [n][T+1] */
+  float* value_preds;      /* [n][T+1] */
+  float* rewards;          /* [n][T+1] */
+  float* masks;            /* [n][T+1] */
+  int32_t* command;        /* [n][T+1] */
+  float* hn;               /* [n][T+1][hidden_size] */
+  float* cn;               /* [n][T+1][hidden_size] */
+  int32_t storages, num_steps, seq_length, feature_dims, hidden_size;
+} cadre_rollout_pool;
+
+/* One act step of E environments into the pool at cursor `slot` (0 <= slot <= num_steps), on an engine with
+ * workers = 1, mini_batch = E: storages_host / indices_host as for cadre_ppo_evaluate (the actor's [E][8][530]
+ * windows and commands; indices must be 0..E-1 for both heads). Runs the forward plan and head_eval_kernel unchanged
+ * (row_out as cadre_ppo_evaluate, fp32 [2][E][36]), then ONE kernel that, for environment e and head h (storage
+ * n = 2e + h), draws a_h with the sampler above (env id env_ids[e], word h, A = 33 / 3) and writes
+ * action[n][slot], action_log_probs[n][slot] = lp_a, value_preds[n][slot], command[n][slot], obs[n][slot] = the
+ * window of e, and, only when slot < num_steps, hn[n][slot+1] / cn[n][slot+1] = hidden_hn / hidden_cn (fp32
+ * [hidden_size], the agent's hidden_state), as RolloutStorage.insert does (storage.py:45-58); actions_out int64
+ * [E][2] receives the draws for one device-to-host copy. The pool needs storages = 2E, seq_length = 8,
+ * feature_dims = hidden_size = 530. */
+int cadre_ppo_act(void* handle, const cadre_storage_ref* storages_host, const int32_t* indices_host,
+                  const float* params, float* row_out, const cadre_rollout_pool* pool, int slot, uint64_t seed,
+                  uint64_t tick, const int32_t* env_ids, const float* hidden_hn, const float* hidden_cn,
+                  int64_t* actions_out, void* stream);
+/* Rewards and masks of slot `slot` of every storage (train.py:60-72: env.step, then insert): two cudaMemcpy2DAsync
+ * from host rows rewards_host / masks_host fp32 [storages] (pinned for an asynchronous copy) into the strided columns
+ * [n][slot]. The caller keeps the host rows unchanged until the stream has consumed them. */
+int cadre_rollout_env_results(const cadre_rollout_pool* pool, int slot, const float* rewards_host,
+                              const float* masks_host, void* stream);
+/* Bootstrap values of all workers in one forward (train.py:76-79, agent.py:143-164) on an engine with
+ * mini_batch = 1: storages_host / indices_host as for cadre_ppo_evaluate (index num_steps of every storage, hn / cn
+ * holding the agent's hidden_state at that index); row_out fp32 [2][workers][36] scratch; next_value fp32
+ * [workers][2] = value of worker w's head h, exactly 0 where bit w of done_mask is set. No host synchronisation. */
+int cadre_ppo_bootstrap(void* handle, const cadre_storage_ref* storages_host, const int32_t* indices_host,
+                        const float* params, float* row_out, uint64_t done_mask, float* next_value, void* stream);
+
+/* ------------------------------------------------------------------------------------------------------
  * Gradient exchange across the ranks of one NVSwitch domain, in place: grads <- sum over ranks, every rank receives
  * the same bits. Replaces Shared_grad_buffers.add_gradient + the chief installing the summed gradient
  * (ppo_agent/models.py:231-239, ppo_agent/chief.py:13-16). The buffer must be symmetric memory: buffer_ptrs_host[r] =
