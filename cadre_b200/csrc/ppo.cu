@@ -215,6 +215,8 @@ struct HeadParams {
   float* losses;        // [W][2][3] value, action, entropy (un-scaled means), written by the last CTA of the grid
   float* partial;       // [E][cap / HEAD_ROWS][HEAD_PARTIAL] per-CTA partial sums (scratch)
   float* loss_e;        // [E][W][3] per-expert loss sums (scratch)
+  float* diag;          // [W][2][4] update diagnostics (see below), written by the last CTA; NULL: not computed
+  float* diag_e;        // [E][W][4] per-expert diagnostics sums (scratch)
   unsigned* ctr;        // [E] finished CTAs per expert, [E] finished experts (zero at launch)
   int cap, W;
   float inv_mb, clip, value_coeff, clip_coeff, ent_coeff;
@@ -222,15 +224,24 @@ struct HeadParams {
 
 constexpr int HEAD_ROWS_PER_CTA = 32;
 constexpr int HEAD_MAX_W = 64;   // workers per engine the loss reduction is sized for
-// per-CTA partial: dW3A [33][128], dW3C [128], dB3A [36], dB3C [4], losses [HEAD_MAX_W][3]
+// per-CTA partial: dW3A [33][128], dW3C [128], dB3A [36], dB3C [4], losses [HEAD_MAX_W][3], diagnostics [HEAD_MAX_W][4]
 constexpr int HP_W3A = 0, HP_W3C = AMAX * HID, HP_B3A = HP_W3C + HID, HP_B3C = HP_B3A + B3A_LD, HP_LOSS = HP_B3C + 4;
-constexpr int HEAD_PARTIAL = HP_LOSS + HEAD_MAX_W * 3;
+constexpr int HP_DIAG = HP_LOSS + HEAD_MAX_W * 3;
+constexpr int HEAD_PARTIAL = HP_DIAG + HEAD_MAX_W * 4;
+// Update diagnostics per worker and head, means over the minibatch (d = lp - old_lp):
+//   [0] approximate KL, expm1(d) - d   [1] old_lp - lp   [2] fraction of rows with |ratio - 1| > clip
+//   [3] fraction of rows with |v - old_v| > clip (the value clip of agent.py:184-193)
+// Per-row terms are summed unweighted through the loss terms' ordered reduction and scaled by 1 / mini_batch once at
+// the end, so the clip fractions are exactly count * (1 / mini_batch).
+constexpr int DIAG_TERMS = 4;
 
 // Every sum of this kernel has a FIXED order (rows of a CTA in sequence, CTAs of an expert by block index, experts of
 // a head by index), so losses and last-layer gradients are bit-reproducible from run to run: each CTA writes its
 // partial sums to scratch, the last CTA of an expert to finish (device-wide counter) reduces them in block order, and
 // the last expert to finish reduces the per-expert losses in expert order. No floating-point atomics.
-__global__ void __launch_bounds__(256) head_kernel(const HeadParams p) {
+// Launched with 256 threads. The register cap is the count the kernel had before the diagnostics terms (ptxas would
+// otherwise take 73; no spills at 72, and 3 CTAs per SM either way).
+__global__ void __maxnreg__(72) head_kernel(const HeadParams p) {
   pdl_trigger();
   pdl_wait();
   const int e = blockIdx.y, head = e >> 2;
@@ -246,6 +257,7 @@ __global__ void __launch_bounds__(256) head_kernel(const HeadParams p) {
   __shared__ float s_dl[HEAD_ROWS_PER_CTA][AMAX + 3];  // d loss / d logits of the CTA's rows
   __shared__ float s_dv[HEAD_ROWS_PER_CTA];
   __shared__ float s_lt[HEAD_ROWS_PER_CTA][3];         // loss terms of the CTA's rows
+  __shared__ float s_dg[HEAD_ROWS_PER_CTA][DIAG_TERMS]; // diagnostics terms of the CTA's rows (p.diag != NULL)
   __shared__ int s_wk[HEAD_ROWS_PER_CTA];              // worker of each row (-1: padding row)
   __shared__ int s_last;
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -345,6 +357,13 @@ __global__ void __launch_bounds__(256) head_kernel(const HeadParams p) {
       s_lt[slot - row0][1] = wgt * action_term;
       s_lt[slot - row0][2] = wgt * ent;
       s_wk[slot - row0] = p.sc.worker[row];
+      if (p.diag) {
+        const float d = lp - old_lp;
+        s_dg[slot - row0][0] = expm1f(d) - d;
+        s_dg[slot - row0][1] = old_lp - lp;
+        s_dg[slot - row0][2] = fabsf(ratio - 1.f) > p.clip ? 1.f : 0.f;
+        s_dg[slot - row0][3] = fabsf(dvv) > p.clip ? 1.f : 0.f;
+      }
     }
     // backward seeds (autograd conventions of torch.min / torch.max / clamp: ties split evenly, clamp passes
     // the gradient on the closed interval)
@@ -428,6 +447,13 @@ __global__ void __launch_bounds__(256) head_kernel(const HeadParams p) {
       for (int r = 0; r < HEAD_ROWS_PER_CTA; ++r)
         if (s_wk[r] == w) l0 += s_lt[r][0], l1 += s_lt[r][1], l2 += s_lt[r][2];
       part[HP_LOSS + w * 3 + 0] = l0, part[HP_LOSS + w * 3 + 1] = l1, part[HP_LOSS + w * 3 + 2] = l2;
+    } else if (p.diag && tid >= 192 && tid < 192 + p.W) {   // diagnostics terms of worker tid - 192, rows in order
+      const int w = tid - 192;
+      float d0 = 0.f, d1 = 0.f, d2 = 0.f, d3 = 0.f;
+      for (int r = 0; r < HEAD_ROWS_PER_CTA; ++r)
+        if (s_wk[r] == w) d0 += s_dg[r][0], d1 += s_dg[r][1], d2 += s_dg[r][2], d3 += s_dg[r][3];
+      float* pd = part + HP_DIAG + w * DIAG_TERMS;
+      pd[0] = d0, pd[1] = d1, pd[2] = d2, pd[3] = d3;
     }
   }
   // ---- phase 3: the last CTA of the expert reduces the partials in block order
@@ -466,6 +492,13 @@ __global__ void __launch_bounds__(256) head_kernel(const HeadParams p) {
     }
     }
   }
+  if (p.diag) {
+    for (int i = tid; i < p.W * DIAG_TERMS; i += 256) {
+      float sum = 0.f;
+      for (int b = 0; b < nblk; ++b) sum += __ldcg(pe + static_cast<long long>(b) * HEAD_PARTIAL + HP_DIAG + i);
+      p.diag_e[e * HEAD_MAX_W * DIAG_TERMS + i] = sum;
+    }
+  }
   // ---- phase 4: the last expert to finish adds the per-expert losses in expert order
   __threadfence();
   __syncthreads();
@@ -483,6 +516,15 @@ __global__ void __launch_bounds__(256) head_kernel(const HeadParams p) {
     for (int x = 0; x < 4; ++x)
       if (p.counts[h * 4 + x] > 0) sum += __ldcg(p.loss_e + (h * 4 + x) * HEAD_MAX_W * 3 + w * 3 + c);
     p.losses[(w * 2 + h) * 3 + c] = sum;
+  }
+  if (p.diag) {
+    for (int i = tid; i < p.W * 2 * DIAG_TERMS; i += 256) {
+      const int w = i / (2 * DIAG_TERMS), h = (i / DIAG_TERMS) % 2, c = i % DIAG_TERMS;
+      float sum = 0.f;
+      for (int x = 0; x < 4; ++x)
+        if (p.counts[h * 4 + x] > 0) sum += __ldcg(p.diag_e + (h * 4 + x) * HEAD_MAX_W * DIAG_TERMS + w * DIAG_TERMS + c);
+      p.diag[i] = sum * p.inv_mb;
+    }
   }
 }
 
@@ -684,7 +726,9 @@ struct PpoPlan {
   __half *WIH16 = nullptr, *WHH16 = nullptr, *WHHT16 = nullptr;   // fp16 weight copies (wcvt_kernel)
   CUtensorMap tmW, tmWT;
   cudaEvent_t ev_wcvt_fork = nullptr, ev_wcvt = nullptr;
-  float *head_partial = nullptr, *head_loss_e = nullptr;   // head_kernel scratch (ordered reductions)
+  float *head_partial = nullptr, *head_loss_e = nullptr, *head_diag_e = nullptr;   // head_kernel scratch (ordered reductions)
+  float* diag_out = nullptr;       // cadre_ppo_set_diagnostics: [W][2][4] of the next update, 16 norms of the next Adam step
+  float* norms_out = nullptr;
   unsigned* seq_sync = nullptr;          // [0, E]: forward counters + error flag, [16, 16 + E]: backward, [32, 32 + E]: head
   CUtensorMap tmH, tmDG;
   float bwd_scale = 1.f;
@@ -757,6 +801,7 @@ static PpoPlan* ppo_create(const cadre_ppo_config* cfg) {
   CADRE_REQUIRE(cfg->workers <= HEAD_MAX_W, "at most 64 workers per engine");
   P->head_partial = dalloc<float>(static_cast<size_t>(E) * (P->cap / HEAD_ROWS_PER_CTA) * HEAD_PARTIAL);
   P->head_loss_e = dalloc<float>(static_cast<size_t>(E) * HEAD_MAX_W * 3);
+  P->head_diag_e = dalloc<float>(static_cast<size_t>(E) * HEAD_MAX_W * DIAG_TERMS);
   {
     const uint64_t dims_h[4] = {(uint64_t)F, (uint64_t)P->cap, 9, (uint64_t)E};
     const uint64_t str_h[3] = {9ull * LS_LDH16 * 2, 1ull * LS_LDH16 * 2, (uint64_t)P->cap * 9 * LS_LDH16 * 2};
@@ -851,7 +896,7 @@ static PpoPlan* ppo_create(const cadre_ppo_config* cfg) {
 
 static void ppo_destroy(PpoPlan* P) {
   if (!P) return;
-  void* ptrs[] = {P->head_partial, P->head_loss_e, P->X16, P->H16, P->G16, P->dG16, P->WIH16, P->WHH16, P->WHHT16, P->seq_sync, P->XP9, P->H8, P->C9, P->Y1, P->Y2, P->dZ1, P->dZ2, P->dH, P->dC, P->bsum,
+  void* ptrs[] = {P->head_partial, P->head_loss_e, P->head_diag_e, P->X16, P->H16, P->G16, P->dG16, P->WIH16, P->WHH16, P->WHHT16, P->seq_sync, P->XP9, P->H8, P->C9, P->Y1, P->Y2, P->dZ1, P->dZ2, P->dH, P->dC, P->bsum,
                   P->sc.action, P->sc.worker, P->sc.old_v, P->sc.ret, P->sc.old_lp, P->sc.adv, P->row_slot,
                   P->row_expert, P->counts, P->counts9, P->idx_dev, P->ctrs, P->xp_tiles, P->refs_dev, P->opt.chunk_off, P->opt.chunk_len,
                   P->opt.chunk_mod, P->opt.mod_first, P->opt.partial, P->opt.clip_coef, P->opt.norms, P->opt.scalars};
@@ -977,6 +1022,7 @@ static void ppo_update(PpoPlan* P, const cadre_storage_ref* refs_host, const int
     hp.Y2 = P->Y2, hp.dZ2 = P->dZ2, hp.params = params, hp.grads = grads, hp.counts = P->counts, hp.sc = P->sc;
     hp.losses = losses, hp.cap = cap, hp.W = W, hp.inv_mb = 1.f / static_cast<float>(mb);
     hp.partial = P->head_partial, hp.loss_e = P->head_loss_e, hp.ctr = P->seq_sync + 32;
+    hp.diag = P->diag_out, hp.diag_e = P->head_diag_e;
     hp.clip = P->cfg.clip, hp.value_coeff = P->cfg.value_coeff, hp.clip_coeff = P->cfg.clip_coeff;
     hp.ent_coeff = P->cfg.ent_coeff;
     launch_k(head_kernel, dim3(dim3(cap / HEAD_ROWS_PER_CTA, E)), dim3(256), 0, s, hp), ++n;
@@ -1203,7 +1249,7 @@ int cadre_ppo_adam_step(void* handle, float* params, const float* grads, float* 
   CADRE_REQUIRE(P && params && grads && exp_avg && exp_avg_sq && step >= 0, "adam_step arguments");
   if (step >= 1) P->host_step = step + 1;   // the one-step update path restarts the device counter from here
   cadre::launch_clip_adam(P->opt, params, grads, exp_avg, exp_avg_sq, max_grad_norm, lr, beta1, beta2, eps, step,
-                          static_cast<cudaStream_t>(stream), 0, 16, P->ctrs + 1);
+                          static_cast<cudaStream_t>(stream), 0, 16, P->ctrs + 1, P->norms_out);
   CADRE_API_END
 }
 
@@ -1253,7 +1299,16 @@ int cadre_ppo_adam_step_modules(void* handle, float* params, const float* grads,
   PpoPlan* P = static_cast<PpoPlan*>(handle);
   CADRE_REQUIRE(P && params && grads && exp_avg && exp_avg_sq && step >= 0, "adam_step arguments");
   cadre::launch_clip_adam(P->opt, params, grads, exp_avg, exp_avg_sq, max_grad_norm, lr, beta1, beta2, eps, step,
-                          static_cast<cudaStream_t>(stream), mod_begin, mod_end, P->ctrs + 1);
+                          static_cast<cudaStream_t>(stream), mod_begin, mod_end, P->ctrs + 1, P->norms_out);
+  CADRE_API_END
+}
+
+int cadre_ppo_set_diagnostics(void* handle, float* diag_out, float* norms_out) {
+  CADRE_API_BEGIN
+  PpoPlan* P = static_cast<PpoPlan*>(handle);
+  CADRE_REQUIRE(P != nullptr, "set_diagnostics: ppo handle is NULL");
+  P->diag_out = diag_out;
+  P->norms_out = norms_out;
   CADRE_API_END
 }
 

@@ -240,7 +240,7 @@ __global__ void __launch_bounds__(256) sqnorm_partial_kernel(const float* __rest
 __global__ void sqnorm_final_kernel(const float* __restrict__ partial, const int* __restrict__ mod_first,
                                     float max_norm, float* __restrict__ clip_coef, float* __restrict__ norms,
                                     int mod_begin, int step, const int* __restrict__ dev_step, float lr, float beta1,
-                                    float beta2, float* __restrict__ scalars) {
+                                    float beta2, float* __restrict__ scalars, float* __restrict__ norms_hist) {
   pdl_trigger();
   pdl_wait();
   // one warp per module; chunks of a module are contiguous in the chunk table
@@ -260,6 +260,7 @@ __global__ void sqnorm_final_kernel(const float* __restrict__ partial, const int
   if (lane == 0) {
     const float total = static_cast<float>(sqrt(s));
     norms[m] = total;
+    if (norms_hist) norms_hist[m] = total;   // per-step history slot (cadre_ppo_set_diagnostics)
     clip_coef[m] = fminf(max_norm / (total + 1e-6f), 1.0f);  // torch.nn.utils.clip_grad_norm_
   }
 }
@@ -301,7 +302,7 @@ __global__ void __launch_bounds__(256) adam_kernel(float* __restrict__ p, const 
 
 void launch_clip_adam(const OptTables& t, float* params, const float* grads, float* m, float* v, float max_norm,
                       float lr, float beta1, float beta2, float eps, int step, cudaStream_t s, int mod_begin,
-                      int mod_end, const int* dev_step) {
+                      int mod_end, const int* dev_step, float* norms_hist) {
   CADRE_REQUIRE(mod_begin >= 0 && mod_begin < mod_end && mod_end <= 16, "module range");
   CADRE_REQUIRE(step >= 1 || dev_step != nullptr, "Adam step");
   // chunks of modules [mod_begin, mod_end) are contiguous in the chunk table (it is sorted by module)
@@ -309,10 +310,56 @@ void launch_clip_adam(const OptTables& t, float* params, const float* grads, flo
   if (nc <= 0) return;
   launch_k(sqnorm_partial_kernel, dim3(nc), dim3(256), 0, s, grads, t.chunk_off + c0, t.chunk_len + c0, t.partial + c0);
   launch_k(sqnorm_final_kernel, dim3(mod_end - mod_begin), dim3(32), 0, s, t.partial, t.mod_first, max_norm, t.clip_coef,
-           t.norms, mod_begin, step, dev_step, lr, beta1, beta2, t.scalars);
+           t.norms, mod_begin, step, dev_step, lr, beta1, beta2, t.scalars, norms_hist);
   launch_k(adam_kernel, dim3(nc), dim3(256), 0, s, params, grads, m, v, t.chunk_off + c0, t.chunk_len + c0, t.chunk_mod + c0,
            t.clip_coef, beta1, beta2, eps, t.scalars);
   CADRE_CUDA_CHECK(cudaGetLastError());
+}
+
+// ---------------------------------------------------------------------------------------------------------
+// Rollout statistics after compute_returns, one warp per (env, head) sequence of T steps, in fp64 with population
+// variances: out[e] = [explained variance 1 - Var(R - V) / Var(R) (NaN when Var(R) = 0, as SB3's explained_variance),
+// mean and std of the raw advantage R - V, mean and std of R, mean of V]. Two passes (means, then centred sums); the
+// second re-reads the sequence from L1 / L2. Lane partial sums are combined with a fixed butterfly: deterministic.
+constexpr int ROLLOUT_STATS = 6;
+__device__ __forceinline__ double warp_sum_f64(double s) {
+  for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+  return s;
+}
+__global__ void __launch_bounds__(256) rollout_stats_kernel(const float* __restrict__ returns,
+                                                            const float* __restrict__ values, int E, int T,
+                                                            float* __restrict__ out) {
+  pdl_trigger();
+  pdl_wait();
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int e = blockIdx.x * (blockDim.x >> 5) + warp;
+  if (e >= E) return;
+  const float* r = returns + static_cast<long long>(e) * (T + 1);
+  const float* v = values + static_cast<long long>(e) * (T + 1);
+  double sr = 0.0, sv = 0.0;
+  for (int i = lane; i < T; i += 32) {
+    sr += static_cast<double>(r[i]);
+    sv += static_cast<double>(v[i]);
+  }
+  const double n = static_cast<double>(T);
+  const double mr = warp_sum_f64(sr) / n, mv = warp_sum_f64(sv) / n, ma = mr - mv;
+  double qr = 0.0, qa = 0.0;
+  for (int i = lane; i < T; i += 32) {
+    const double rr = static_cast<double>(r[i]);
+    const double dr = rr - mr, da = (rr - static_cast<double>(v[i])) - ma;
+    qr += dr * dr;
+    qa += da * da;
+  }
+  const double var_r = warp_sum_f64(qr) / n, var_a = warp_sum_f64(qa) / n;
+  if (lane == 0) {
+    float* o = out + static_cast<long long>(e) * ROLLOUT_STATS;
+    o[0] = var_r == 0.0 ? __int_as_float(0x7fc00000) : static_cast<float>(1.0 - var_a / var_r);
+    o[1] = static_cast<float>(ma);
+    o[2] = static_cast<float>(sqrt(var_a));
+    o[3] = static_cast<float>(mr);
+    o[4] = static_cast<float>(sqrt(var_r));
+    o[5] = static_cast<float>(mv);
+  }
 }
 
 }  // namespace cadre
@@ -390,6 +437,16 @@ int cadre_gae(const float* rewards, float* values, const float* masks, const flo
   if (smem > 48 * 1024) cadre::ensure_dynamic_smem(kern, smem, configured[which]);
   cadre::launch_k(kern, dim3((E + warps - 1) / warps), dim3(warps * 32), smem, static_cast<cudaStream_t>(stream),
                   rewards, values, masks, next_value, returns, adv, E, T, gamma, tau, normalize);
+  CADRE_CUDA_CHECK(cudaGetLastError());
+  CADRE_API_END
+}
+
+int cadre_rollout_stats(const float* returns, const float* values, int E, int T, float* out, void* stream) {
+  CADRE_API_BEGIN
+  CADRE_REQUIRE(returns && values && out, "rollout_stats pointers");
+  CADRE_REQUIRE(E > 0 && T > 0, "rollout_stats sizes (E > 0, T > 0)");
+  cadre::launch_k(cadre::rollout_stats_kernel, dim3((E + 7) / 8), dim3(256), 0, static_cast<cudaStream_t>(stream),
+                  returns, values, E, T, out);
   CADRE_CUDA_CHECK(cudaGetLastError());
   CADRE_API_END
 }

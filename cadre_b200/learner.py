@@ -95,10 +95,21 @@ class RolloutPool:
                  self.next_value, b["returns"].view(n, T + 1), b["advantages"].view(n, T), self.gamma, self.tau,
                  normalize)
 
+    def rollout_stats(self):
+        """Statistics of every storage's returns and values after `compute_returns`, one launch and one synchronisation:
+        {name: float32 [W, 2]} for the names of ppo.ROLLOUT_STATS (explained variance, NaN where the returns are
+        constant; mean / std of the raw advantage R - V; mean / std of the returns; mean of the values)."""
+        n, T = self.workers * 2, self.num_steps
+        b = self.batched
+        out = _ppo.rollout_stats(b["returns"].view(n, T + 1), b["value_preds"].view(n, T + 1)).cpu().numpy()
+        return {name: out[:, k].reshape(self.workers, 2) for k, name in enumerate(_ppo.ROLLOUT_STATS)}
+
 
 class Learner:
     def __init__(self, workers, mini_batch, ppo_state, device="cuda:0", clip=0.1, value_coeff=0.1, clip_coeff=1.0,
-                 ent_coeff=0.01, lr=3e-4, max_grad_norm=250.0, process_group=None, seeds=None):
+                 ent_coeff=0.01, lr=3e-4, max_grad_norm=250.0, process_group=None, seeds=None, diagnostics=False):
+        """`diagnostics`: record, for every update step, the approximate KL, clip fractions and pre-clip module gradient
+        norms in device-side histories (no host synchronisation inside a phase); read them with `diagnostics()`."""
         self.device = torch.device(device)
         self.workers, self.mini_batch = workers, mini_batch
         self.value_coeff, self.clip_coeff, self.ent_coeff = value_coeff, clip_coeff, ent_coeff
@@ -140,6 +151,8 @@ class Learner:
         self.loss_sum = torch.zeros(workers, 2, 3, device=self.device)     # summed over the update steps of learn()
         self.loss_steps = 0
         self.step_count = 0
+        self.diagnostics_on = bool(diagnostics)
+        self._diag_hist = self._norm_hist = None      # [steps, W, 2, 4] and [steps, 16] of the last learn() / update_step
         self.pg = process_group
         self.overlap_allreduce = os.environ.get("CADRE_NO_ALLREDUCE_OVERLAP", "0") != "1"
         self._comm_stream = None
@@ -243,9 +256,11 @@ class Learner:
         advs = [(s.advantages, t.advantages) for s, t in storages]
         if self.world > 1 and self._comm_stream is None:
             self._setup_pipeline()
+        self._diag_step(0, 1)
         self.engine.update(storages, advs, indices, self.params, self.grads, self.losses)
         self.step_count += 1
         self._exchange_and_step(self.step_count)
+        self._diag_step(None)
         return self.losses if async_losses else self.scaled_losses()
 
     def scaled_losses(self, mean=False):
@@ -273,13 +288,53 @@ class Learner:
         while n < idx_all.shape[0]:                       # (the staging table holds 64 steps)
             m = min(64, idx_all.shape[0] - n)
             self.engine.stage(storages, advs, idx_all[n:n + m], self.step_count + 1)
-            for _ in range(m):
+            for k in range(m):
+                self._diag_step(n + k, idx_all.shape[0])
                 self.engine.update_staged(self.params, self.grads, self.losses)
                 self._exchange_and_step(0)
                 self.step_count += 1
             n += m
+        self._diag_step(None)
         self.loss_steps = idx_all.shape[0]
         return idx_all.shape[0]
+
+    # ---------------------------------------------------------------- diagnostics
+    def _diag_step(self, k, steps=None):
+        """With diagnostics on: point the engine at row k of histories of `steps` update steps (new histories when k is
+        0); k = None detaches them. Only host-side pointers change, so this costs no synchronisation."""
+        if not self.diagnostics_on:
+            return
+        if k is None:
+            self.engine.set_diagnostics(None, None)
+            return
+        if k == 0:
+            self._diag_hist = torch.zeros(steps, self.workers, 2, len(_ppo.DIAG_TERMS), device=self.device)
+            self._norm_hist = torch.zeros(steps, 16, device=self.device)
+        self.engine.set_diagnostics(self._diag_hist[k], self._norm_hist[k])
+
+    def diagnostics(self):
+        """Diagnostics of the update steps of the last `learn()` (or of the last `update_step`), one synchronisation.
+        Per local worker and head, [steps, W, 2]: `approx_kl` (mean of expm1(d) - d, d = log-prob - old log-prob),
+        `kl_k1` (mean of -d), `clip_frac` (rows with |ratio - 1| > clip) and `value_clip_frac` (rows with
+        |value - old value| > clip); [steps, 16]: `grad_norm`, every module's gradient norm before clipping (after the
+        all-reduce, so the same on every rank), columns in `modules` order (the reference's model_dict order), and
+        `grad_clipped` = grad_norm > max_grad_norm."""
+        if not self.diagnostics_on:
+            raise CadreError("diagnostics() needs Learner(..., diagnostics=True)")
+        if self._diag_hist is None:
+            raise CadreError("diagnostics(): no update step has run yet")
+        steps = self._diag_hist.shape[0]
+        flat = torch.cat([self._diag_hist.reshape(-1), self._norm_hist.reshape(-1)]).cpu().numpy()
+        d = flat[:self._diag_hist.numel()].reshape(self._diag_hist.shape)
+        norms = flat[self._diag_hist.numel():].reshape(steps, 16)
+        modules = list(ppo_params.MODULE_ORDER)
+        # engine module ids: e = LSTM of expert e, 8 + e = actor-critic of expert e (expert = head * 4 + command)
+        cols = [ppo_params.expert_of(m) + (0 if "_lstm_" in m else 8) for m in modules]
+        out = {name: d[..., i] for i, name in enumerate(_ppo.DIAG_TERMS)}
+        out["grad_norm"] = norms[:, cols]
+        out["grad_clipped"] = out["grad_norm"] > self.max_grad_norm
+        out["modules"] = modules
+        return out
 
     def check(self):
         """Synchronise and raise CadreError if a bounded wait inside a kernel (LSTM hand-off, all-reduce barrier) ever

@@ -30,6 +30,8 @@ class RolloutPoolC(ctypes.Structure):
 
 
 ROW_OUT = 36
+DIAG_TERMS = ("approx_kl", "kl_k1", "clip_frac", "value_clip_frac")      # last axis of the update diagnostics
+ROLLOUT_STATS = ("explained_variance", "adv_mean", "adv_std", "return_mean", "return_std", "value_mean")
 
 
 def _check_tensor(t, dtype, name):
@@ -200,6 +202,18 @@ class PpoEngine:
                 ctypes.c_float(max_grad_norm), ctypes.c_float(lr), ctypes.c_float(betas[0]), ctypes.c_float(betas[1]),
                 ctypes.c_float(eps), int(step), int(mod_begin), int(mod_end), _lib.stream_ptr(self.device)))
 
+    def set_diagnostics(self, diag=None, norms=None):
+        """Destinations of the update diagnostics (cadre_ppo_set_diagnostics): every later `update*` writes `diag` fp32
+        [W, 2, 4] (DIAG_TERMS per worker and head) and every later `adam_step*` writes the pre-clip norms of the modules
+        it steps into `norms` fp32 [16]. None turns either off. The tensors must stay alive while they are set."""
+        for t, n, name in ((diag, self.workers * 2 * len(DIAG_TERMS), "diag"), (norms, 16, "norms")):
+            if t is not None:
+                _check_tensor(t, torch.float32, name)
+                if t.numel() != n or (self.device.index is not None and t.device.index != self.device.index):
+                    raise _lib.CadreError(f"set_diagnostics: `{name}` must hold {n} floats on {self.device} "
+                                          f"(got {t.numel()} on {t.device})")
+        _lib.check(self._lib.cadre_ppo_set_diagnostics(self._h, _lib.ptr(diag), _lib.ptr(norms)))
+
     def check(self):
         """Synchronise and raise CadreError if a recurrence kernel of an earlier call timed out on a hand-off."""
         with torch.cuda.device(self.device):
@@ -236,3 +250,24 @@ def gae(rewards, values, masks, next_value, returns, adv, gamma=0.99, tau=0.95, 
                                         _lib.ptr(returns), _lib.ptr(adv), E, T1 - 1, ctypes.c_float(gamma),
                                         ctypes.c_float(tau), int(bool(normalize)), _lib.stream_ptr(rewards.device)))
     return returns, adv
+
+
+def rollout_stats(returns, values, out=None):
+    """cadre_rollout_stats over E sequences: returns / values fp32 [E, T+1] after `gae` (steps t < T are used). Returns
+    out fp32 [E, 6] = ROLLOUT_STATS: explained variance (NaN where Var(R) = 0), mean and std of R - V, mean and std of
+    R, mean of V (fp64 sums, population variances)."""
+    for t, name in ((returns, "returns"), (values, "values")):
+        _check_tensor(t, torch.float32, name)
+        if t.dim() != 2 or t.shape != returns.shape or t.shape[1] < 2:
+            raise _lib.CadreError(f"rollout_stats: `{name}` must be [E, T+1] with T >= 1 like `returns` "
+                                  f"(got {tuple(t.shape)})")
+    E, T = returns.shape[0], returns.shape[1] - 1
+    if out is None:
+        out = torch.empty(E, len(ROLLOUT_STATS), device=returns.device, dtype=torch.float32)
+    _check_tensor(out, torch.float32, "out")
+    if out.shape != (E, len(ROLLOUT_STATS)):
+        raise _lib.CadreError(f"rollout_stats: `out` must be [{E}, {len(ROLLOUT_STATS)}] (got {tuple(out.shape)})")
+    with torch.cuda.device(returns.device):
+        _lib.check(_lib.lib().cadre_rollout_stats(_lib.ptr(returns), _lib.ptr(values), E, T, _lib.ptr(out),
+                                                  _lib.stream_ptr(returns.device)))
+    return out

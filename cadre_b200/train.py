@@ -16,7 +16,7 @@ from .synthetic_env import SyntheticEnv
 
 
 def train(rank, train_cfg, agent_cfg, env_cfg, rollout_cfg, danet_state, ppo_state=None, workers=1, max_episode=None,
-          process_group=None, log=print, batched_acting=True, device_rollout=False):
+          process_group=None, log=print, batched_acting=True, device_rollout=False, diagnostics=False):
     """One rank: `workers` logical workers (env + rollout pair each) sharing one agent replica. With
     `batched_acting` the rank's workers are stepped together through `BatchedActor` (one encoder batch of the newest
     frames + one routed LSTM / head evaluation per tick) instead of one `agent.act` call per worker.
@@ -24,7 +24,10 @@ def train(rank, train_cfg, agent_cfg, env_cfg, rollout_cfg, danet_state, ppo_sta
     pool with a fixed number of launches and copies (`BatchedActor.act_into`, `RolloutPool.write_env_results`), and
     bootstraps all workers' values in one forward (`BatchedActor.bootstrap_into`). Its draws come from a counter-based
     generator keyed by (env seed, worker id, tick), not from torch's RNG, so its trajectories differ from the default
-    path's."""
+    path's.
+    `diagnostics` records the PPO update diagnostics of every episode (`Learner.diagnostics`, `RolloutPool.rollout_stats`):
+    each `history` entry gains a dict of them as a fourth element, and rank 0 logs one more line per `log_interval`.
+    Values are those of this rank's workers. Training itself is unchanged."""
     if device_rollout and not batched_acting:
         raise ValueError("device_rollout=True needs batched_acting=True")
     device = torch.device("cuda:" + str(agent_cfg.model_cfg.device_num))
@@ -37,7 +40,8 @@ def train(rank, train_cfg, agent_cfg, env_cfg, rollout_cfg, danet_state, ppo_sta
     agent = CadreAgent(**dict(agent_cfg, rank=rank), danet_state=danet_state, ppo_state=ppo_state, mini_batch=mb)
     learner = Learner(workers, mb, ppo_state, device, agent_cfg.clip, agent_cfg.value_coeff, agent_cfg.clip_coeff,
                       agent_cfg.ent_coeff, train_cfg.lr, train_cfg.max_grad_norm, process_group,
-                      seeds=[env_cfg.get("seed", 0) + rank * workers + w for w in range(workers)])
+                      seeds=[env_cfg.get("seed", 0) + rank * workers + w for w in range(workers)],
+                      diagnostics=diagnostics)
     agent.owner.params = learner.params          # the acting replica reads the learner's parameters directly
     pool = RolloutPool(workers, dict(rollout_cfg, hidden_size=hidden_size), device)
     obs = [e.reset() for e in envs]
@@ -75,9 +79,26 @@ def train(rank, train_cfg, agent_cfg, env_cfg, rollout_cfg, danet_state, ppo_sta
         learner.learn(pool, train_cfg.ppo_epoch)                          # train.py:93-110
         L = learner.scaled_losses(mean=True).mean(0)     # mean over update steps and workers
         history.append(L.tolist())
+        if diagnostics:
+            diag = dict(learner.diagnostics(), **pool.rollout_stats())
+            history[-1].append(diag)
         if episode % train_cfg.log_interval == 0 and rank == 0:
             log("Episode: {}, value loss: {:.4f}, policy loss: {:.4f}, entropy loss: {:.4f}".format(episode, *L))
+            if diagnostics:
+                log(_diagnostics_line(episode, diag))
     return learner, history
+
+
+def _diagnostics_line(episode, d):
+    """One log line: per head (steer / throttle) the mean approximate KL and clip fraction over the phase's update steps
+    and the workers, the explained variance (mean over workers), and the largest module gradient norm of the phase with
+    the number of modules clipped in at least one step."""
+    kl, cf = d["approx_kl"].mean((0, 1)), d["clip_frac"].mean((0, 1))
+    ev = [np.nanmean(c) if np.isfinite(c).any() else np.nan for c in d["explained_variance"].T]
+    return ("Episode: {}, approx kl: {:.2e} / {:.2e}, clip fraction: {:.3f} / {:.3f}, explained variance: {:.3f} / {:.3f}, "
+            "max grad norm: {:.2f}, modules clipped: {} of 16".format(
+                episode, kl[0], kl[1], cf[0], cf[1], ev[0], ev[1], d["grad_norm"].max(),
+                int(d["grad_clipped"].any(0).sum())))
 
 
 def _device_rollout(actor, agent, envs, pool, obs, done, num_steps):

@@ -157,6 +157,11 @@ int cadre_encoder_launches(void* handle);
  * values[e][T] is overwritten with next_value[e] exactly as the reference does. */
 int cadre_gae(const float* rewards, float* values, const float* masks, const float* next_value, float* returns,
               float* adv, int E, int T, float gamma, float tau, int normalize, void* stream);
+/* Rollout statistics of E sequences after cadre_gae, over steps t < T of returns / values fp32 [E][T+1] (the raw
+ * advantage R - V is recomputed from them: returns = gae + values). out fp32 [E][6] = explained variance
+ * 1 - Var(R - V) / Var(R) (NaN when Var(R) = 0), mean and std of R - V, mean and std of R, mean of V; fp64 sums,
+ * population variances. One warp per sequence; E > 0, T > 0. */
+int cadre_rollout_stats(const float* returns, const float* values, int E, int T, float* out, void* stream);
 
 /* Sliding-window assembly of rollout observations (env_wrapper.py:900-914 stacks the last `seq_length` frames per
  * tick; train.py:69-72 inserts that window into the steer AND the throttle storage). unique_feats: fp32
@@ -240,6 +245,15 @@ int cadre_ppo_adam_step_modules(void* handle, float* params, const float* grads,
  * bounded so that a lost signal can never hang the GPU). */
 int cadre_ppo_check(void* handle);
 int cadre_ppo_launches(void* handle);
+/* Update diagnostics (off by default). While diag_out is set, each cadre_ppo_update also writes diag_out fp32
+ * [workers][2][4], means over the minibatch of worker w's head h with d = lp - old_lp: [0] approximate KL
+ * expm1(d) - d, [1] old_lp - lp, [2] fraction of rows with |ratio - 1| > clip, [3] fraction of rows with
+ * |v - old_v| > clip; bit-reproducible, no float atomics. While norms_out is set, each cadre_ppo_adam_step* also writes
+ * the pre-clip gradient norm of every module it steps into norms_out[module] (fp32 [16], module order of
+ * cadre_ppo_module_norms). Both are device pointers read at launch time: the host points them at the next row of a
+ * device-side history before each staged step, which needs no synchronisation. NULL turns either off; losses,
+ * gradients and parameters do not depend on the setting. */
+int cadre_ppo_set_diagnostics(void* handle, float* diag_out, float* norms_out);
 
 /* ------------------------------------------------------------------------------------------------------
  * Device-side rollout collection: replaces the host-side Categorical draw (ppo_agent/distributions.py:96-99,
