@@ -223,9 +223,11 @@ inline void ensure_dynamic_smem(Kern kern, size_t smem, size_t* flags) {
   }
 }
 
-// modules [mod_begin, mod_end) only (module e < 8: LSTM of expert e, 8 + e: actor-critic of expert e)
+// modules [mod_begin, mod_end) only (module e < 8: LSTM of expert e, 8 + e: actor-critic of expert e). `gate` (NULL:
+// always step): two device words read at run time, gate[0] != 0 skips the norms and the step, gate[1] != 0 the step only.
 void launch_clip_adam(const OptTables& t, float* params, const float* grads, float* m, float* v, float max_norm,
                       float lr, float beta1, float beta2, float eps, int step, cudaStream_t s, int mod_begin = 0,
-                      int mod_end = 16, const int* dev_step = nullptr, float* norms_hist = nullptr);
+                      int mod_end = 16, const int* dev_step = nullptr, float* norms_hist = nullptr,
+                      const int* gate = nullptr);
 
 }  // namespace cadre

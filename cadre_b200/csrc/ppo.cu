@@ -47,13 +47,20 @@ struct StorageRef {  // == cadre_storage_ref
 // Minibatch indices live in a staged device table [steps][W][2][mb]; the update reads slice `*step_ctr`, which the
 // update's own prep_kernel advances afterwards. A sequence of update steps therefore needs no host-to-device copy
 // between steps and can be replayed from a CUDA graph (cadre_ppo_stage / cadre_ppo_update with indices_host = NULL).
+// `stop` (NULL unless target-KL early stopping is on): once the phase is stopped, every expert gets zero rows, and every
+// later kernel of the update sizes its work from these counts, so the remaining steps of the phase do almost nothing.
 __global__ void __launch_bounds__(1024) route_kernel(const StorageRef* __restrict__ refs,
                                                      const int* __restrict__ idx_all,
                                                      const int* __restrict__ step_ctr, int W, int mb,
                                                      int* __restrict__ row_slot, int* __restrict__ row_expert,
-                                                     int* __restrict__ counts, int* __restrict__ counts9) {
+                                                     int* __restrict__ counts, int* __restrict__ counts9,
+                                                     const int* __restrict__ stop) {
   pdl_trigger();
   pdl_wait();
+  if (stop && *stop) {
+    if (threadIdx.x < 4) counts[blockIdx.x * 4 + threadIdx.x] = 0, counts9[blockIdx.x * 4 + threadIdx.x] = 0;
+    return;
+  }
   const int* idx = idx_all + static_cast<long long>(*step_ctr) * 2 * W * mb;
   __shared__ int base[4];
   __shared__ int wcnt[32][4];
@@ -113,9 +120,11 @@ __global__ void __launch_bounds__(256) pack_kernel(const StorageRef* __restrict_
                                                    const int* __restrict__ row_slot,
                                                    const int* __restrict__ row_expert,
                                                    __half* __restrict__ X16, float* __restrict__ C9,
-                                                   __half* __restrict__ H16, RowScalars sc) {
+                                                   __half* __restrict__ H16, RowScalars sc,
+                                                   const int* __restrict__ stop) {
   pdl_trigger();
   pdl_wait();
+  if (stop && *stop) return;   // no routed rows (route_kernel)
   const int r = blockIdx.x, h = blockIdx.y, R = W * mb;
   const int* idx = idx_all + static_cast<long long>(*step_ctr) * 2 * R;
   const int w = r / mb, i = r - w * mb;
@@ -217,6 +226,7 @@ struct HeadParams {
   float* loss_e;        // [E][W][3] per-expert loss sums (scratch)
   float* diag;          // [W][2][4] update diagnostics (see below), written by the last CTA; NULL: not computed
   float* diag_e;        // [E][W][4] per-expert diagnostics sums (scratch)
+  float* kl_sum;        // [2] per head, the sum over workers of diag[w][h][0] in worker order; NULL: not written
   unsigned* ctr;        // [E] finished CTAs per expert, [E] finished experts (zero at launch)
   int cap, W;
   float inv_mb, clip, value_coeff, clip_coeff, ent_coeff;
@@ -525,6 +535,14 @@ __global__ void __maxnreg__(72) head_kernel(const HeadParams p) {
         if (p.counts[h * 4 + x] > 0) sum += __ldcg(p.diag_e + (h * 4 + x) * HEAD_MAX_W * DIAG_TERMS + w * DIAG_TERMS + c);
       p.diag[i] = sum * p.inv_mb;
     }
+    if (p.kl_sum) {     // this rank's share of the target-KL decision (kl_gate_kernel)
+      __syncthreads();
+      if (tid < 2) {
+        float s = 0.f;
+        for (int w = 0; w < p.W; ++w) s += p.diag[(w * 2 + tid) * DIAG_TERMS];
+        p.kl_sum[tid] = s;
+      }
+    }
   }
 }
 
@@ -708,7 +726,46 @@ __global__ void __launch_bounds__(256) wcvt_kernel(const float* __restrict__ par
 
 __global__ void set_counters_kernel(int* ctrs, int step_ctr, int opt_step) {
   ctrs[0] = step_ctr;
-  ctrs[1] = opt_step;
+  if (opt_step >= 0) ctrs[1] = opt_step;   // opt_step < 0: the Adam step continues from the device counter
+}
+
+// ------------------------------------------------------------------------------------------ target-KL early stopping
+// SB3's rule (on_policy ppo.py: `if approx_kl_div > 1.5 * target_kl: continue_training = False; break`, before the
+// optimizer step) applied on the device, so that a phase of staged update steps needs no host synchronisation. State
+// words of the phase (cadre_ppo_kl_begin clears them):
+constexpr int KS_SKIP_NORM = 0;    // the phase was stopped before the current step: no gradient norms, no Adam step
+constexpr int KS_STOPPED = 1;      // the phase is stopped: no Adam step from the current step on
+constexpr int KS_STEP = 2;         // update steps of the phase gated so far
+constexpr int KS_RUN = 3;          // steps that ran their forward and backward: applied ones + the one that stopped
+constexpr int KS_APPLIED = 4;      // steps whose Adam update was applied
+constexpr int KS_STOPPED_AT = 5;   // index of the step that stopped the phase (valid while KS_STOPPED is set)
+constexpr int KS_WORDS = 8;
+constexpr int KL_HIST_CAP = 4096;  // steps of a phase whose KL is kept
+// One thread, after the cross-rank sum of head_kernel's per-head KL sums and before the step's first norm / Adam
+// launch. KL = sum over heads of (sum over the workers of all ranks) * (1 / total workers), the same operations in the
+// same order on every rank, so every rank takes the same decision from the same bits. A step that is not applied gives
+// back the Adam step prep_kernel took for it.
+__global__ void kl_gate_kernel(const float* __restrict__ kl_sum, float inv_total, float limit, int* __restrict__ st,
+                               float* __restrict__ hist, int* __restrict__ opt_step) {
+  pdl_trigger();
+  pdl_wait();
+  const int n = st[KS_STEP];
+  st[KS_STEP] = n + 1;
+  st[KS_SKIP_NORM] = st[KS_STOPPED];
+  if (st[KS_STOPPED]) {
+    *opt_step -= 1;
+    return;
+  }
+  const float kl = __fadd_rn(__fmul_rn(kl_sum[0], inv_total), __fmul_rn(kl_sum[1], inv_total));
+  if (n < KL_HIST_CAP) hist[n] = kl;
+  st[KS_RUN] += 1;
+  if (kl > limit) {
+    st[KS_STOPPED] = 1;
+    st[KS_STOPPED_AT] = n;
+    *opt_step -= 1;
+  } else {
+    st[KS_APPLIED] += 1;
+  }
 }
 
 // ------------------------------------------------------------------------------------------ plan
@@ -729,6 +786,12 @@ struct PpoPlan {
   float *head_partial = nullptr, *head_loss_e = nullptr, *head_diag_e = nullptr;   // head_kernel scratch (ordered reductions)
   float* diag_out = nullptr;       // cadre_ppo_set_diagnostics: [W][2][4] of the next update, 16 norms of the next Adam step
   float* norms_out = nullptr;
+  // target-KL early stopping (cadre_ppo_set_target_kl): kl_sum = caller's rank-summed [2] (NULL: off)
+  float* kl_sum = nullptr;
+  float kl_limit = 0.f, kl_inv_total = 0.f;
+  int* kl_state = nullptr;         // [KS_WORDS] phase state (kl_gate_kernel)
+  float* kl_hist = nullptr;        // [KL_HIST_CAP] KL of each step of the phase that ran
+  float* kl_diag = nullptr;        // [W][2][4] diagnostics scratch while diag_out is NULL
   unsigned* seq_sync = nullptr;          // [0, E]: forward counters + error flag, [16, 16 + E]: backward, [32, 32 + E]: head
   CUtensorMap tmH, tmDG;
   float bwd_scale = 1.f;
@@ -802,6 +865,9 @@ static PpoPlan* ppo_create(const cadre_ppo_config* cfg) {
   P->head_partial = dalloc<float>(static_cast<size_t>(E) * (P->cap / HEAD_ROWS_PER_CTA) * HEAD_PARTIAL);
   P->head_loss_e = dalloc<float>(static_cast<size_t>(E) * HEAD_MAX_W * 3);
   P->head_diag_e = dalloc<float>(static_cast<size_t>(E) * HEAD_MAX_W * DIAG_TERMS);
+  P->kl_state = dalloc<int>(KS_WORDS);
+  P->kl_hist = dalloc<float>(KL_HIST_CAP);
+  P->kl_diag = dalloc<float>(static_cast<size_t>(cfg->workers) * 2 * DIAG_TERMS);
   {
     const uint64_t dims_h[4] = {(uint64_t)F, (uint64_t)P->cap, 9, (uint64_t)E};
     const uint64_t str_h[3] = {9ull * LS_LDH16 * 2, 1ull * LS_LDH16 * 2, (uint64_t)P->cap * 9 * LS_LDH16 * 2};
@@ -899,7 +965,8 @@ static void ppo_destroy(PpoPlan* P) {
   void* ptrs[] = {P->head_partial, P->head_loss_e, P->head_diag_e, P->X16, P->H16, P->G16, P->dG16, P->WIH16, P->WHH16, P->WHHT16, P->seq_sync, P->XP9, P->H8, P->C9, P->Y1, P->Y2, P->dZ1, P->dZ2, P->dH, P->dC, P->bsum,
                   P->sc.action, P->sc.worker, P->sc.old_v, P->sc.ret, P->sc.old_lp, P->sc.adv, P->row_slot,
                   P->row_expert, P->counts, P->counts9, P->idx_dev, P->ctrs, P->xp_tiles, P->refs_dev, P->opt.chunk_off, P->opt.chunk_len,
-                  P->opt.chunk_mod, P->opt.mod_first, P->opt.partial, P->opt.clip_coef, P->opt.norms, P->opt.scalars};
+                  P->opt.chunk_mod, P->opt.mod_first, P->opt.partial, P->opt.clip_coef, P->opt.norms, P->opt.scalars,
+                  P->kl_state, P->kl_hist, P->kl_diag};
   for (void* p : ptrs) cudaFree(p);
   if (P->side) cudaStreamDestroy(P->side);
   if (P->idx_pinned) cudaFreeHost(P->idx_pinned);
@@ -922,7 +989,7 @@ static GemmArgs tf32_gemm(int a_mn, int b_mn) {
 }
 
 // Upload the storage references and the minibatch indices of `n_steps` consecutive update steps ([n_steps][W][2][mb])
-// and rewind the step counter; `first_step` is the 1-based Adam step of the first of them.
+// and rewind the step counter; `first_step` is the 1-based Adam step of the first of them (0: continue the device counter).
 static void ppo_stage(PpoPlan* P, const cadre_storage_ref* refs_host, const int32_t* idx_host, int n_steps,
                       int first_step, cudaStream_t s) {
   CADRE_REQUIRE(n_steps >= 1 && n_steps <= MAX_STAGED, "between 1 and 64 update steps can be staged");
@@ -942,7 +1009,7 @@ static void ppo_stage(PpoPlan* P, const cadre_storage_ref* refs_host, const int3
 // routing + gather + forward through the second hidden layer (Y2); returns the number of kernels launched.
 // idx_host == nullptr: use the staged table (no host copies: capturable in a CUDA graph).
 static int ppo_forward(PpoPlan* P, const cadre_storage_ref* refs_host, const int32_t* idx_host,
-                       const float* params, cudaStream_t s) {
+                       const float* params, cudaStream_t s, const int* stop = nullptr) {
   const int W = P->cfg.workers, mb = P->cfg.mini_batch, cap = P->cap, R = P->R;
   const long long rs9G = static_cast<long long>(cap) * 9 * G;
   int n = 0;
@@ -959,9 +1026,9 @@ static int ppo_forward(PpoPlan* P, const cadre_storage_ref* refs_host, const int
   CADRE_CUDA_CHECK(cudaMemsetAsync(P->seq_sync + 32, 0, sizeof(unsigned) * (E + 1), s));  // head_kernel reductions
   if (idx_host != nullptr) ppo_stage(P, refs_host, idx_host, 1, P->host_step, s);   // one-step table
   launch_k(route_kernel, dim3(2), dim3(1024), 0, s, P->refs_dev, P->idx_dev, P->ctrs, W, mb, P->row_slot, P->row_expert,
-           P->counts, P->counts9), ++n;
+           P->counts, P->counts9, stop), ++n;
   launch_k(pack_kernel, dim3(dim3(R, 2)), dim3(256), 0, s, P->refs_dev, P->idx_dev, P->ctrs, W, mb, cap, P->row_slot, P->row_expert,
-                                         P->X16, P->C9, P->H16, P->sc), ++n;
+                                         P->X16, P->C9, P->H16, P->sc, stop), ++n;
   launch_k(prep_kernel, dim3((E * G + 255) / 256), dim3(256), 0, s, params, P->bsum, E * G,
            P->counts9, P->xp_tiles, P->xp_max_tiles, P->dG16, cap, P->ctrs, P->ctrs + 1), ++n;
   CADRE_CUDA_CHECK(cudaGetLastError());
@@ -1016,13 +1083,19 @@ static void ppo_update(PpoPlan* P, const cadre_storage_ref* refs_host, const int
   const int W = P->cfg.workers, mb = P->cfg.mini_batch, cap = P->cap;
   CADRE_CUDA_CHECK(cudaMemsetAsync(losses, 0, sizeof(float) * W * 2 * 3, s));
   CADRE_CUDA_CHECK(cudaMemsetAsync(grads + OFF_W3A, 0, sizeof(float) * (TOTAL - OFF_W3A), s));
-  int n = ppo_forward(P, refs_host, idx_host, params, s);
+  // target-KL early stopping applies to staged steps (a phase); a one-step update runs as with it off
+  const bool gate = P->kl_sum != nullptr && idx_host == nullptr;
+  int n = ppo_forward(P, refs_host, idx_host, params, s, gate ? P->kl_state + KS_STOPPED : nullptr);
   {
     HeadParams hp;
     hp.Y2 = P->Y2, hp.dZ2 = P->dZ2, hp.params = params, hp.grads = grads, hp.counts = P->counts, hp.sc = P->sc;
     hp.losses = losses, hp.cap = cap, hp.W = W, hp.inv_mb = 1.f / static_cast<float>(mb);
     hp.partial = P->head_partial, hp.loss_e = P->head_loss_e, hp.ctr = P->seq_sync + 32;
-    hp.diag = P->diag_out, hp.diag_e = P->head_diag_e;
+    hp.diag = P->diag_out, hp.diag_e = P->head_diag_e, hp.kl_sum = nullptr;
+    if (gate) {
+      if (hp.diag == nullptr) hp.diag = P->kl_diag;
+      hp.kl_sum = P->kl_sum;
+    }
     hp.clip = P->cfg.clip, hp.value_coeff = P->cfg.value_coeff, hp.clip_coeff = P->cfg.clip_coeff;
     hp.ent_coeff = P->cfg.ent_coeff;
     launch_k(head_kernel, dim3(dim3(cap / HEAD_ROWS_PER_CTA, E)), dim3(256), 0, s, hp), ++n;
@@ -1159,7 +1232,7 @@ int cadre_ppo_destroy(void* handle) {
 int cadre_ppo_stage(void* handle, const cadre_storage_ref* storages_host, const int32_t* indices_host, int n_steps,
                     int first_adam_step, void* stream) {
   CADRE_API_BEGIN
-  CADRE_REQUIRE(handle && storages_host && indices_host && first_adam_step >= 1, "ppo_stage arguments");
+  CADRE_REQUIRE(handle && storages_host && indices_host && first_adam_step >= 0, "ppo_stage arguments");
   cadre::ppo_stage(static_cast<PpoPlan*>(handle), storages_host, indices_host, n_steps, first_adam_step,
                    static_cast<cudaStream_t>(stream));
   CADRE_API_END
@@ -1249,7 +1322,8 @@ int cadre_ppo_adam_step(void* handle, float* params, const float* grads, float* 
   CADRE_REQUIRE(P && params && grads && exp_avg && exp_avg_sq && step >= 0, "adam_step arguments");
   if (step >= 1) P->host_step = step + 1;   // the one-step update path restarts the device counter from here
   cadre::launch_clip_adam(P->opt, params, grads, exp_avg, exp_avg_sq, max_grad_norm, lr, beta1, beta2, eps, step,
-                          static_cast<cudaStream_t>(stream), 0, 16, P->ctrs + 1, P->norms_out);
+                          static_cast<cudaStream_t>(stream), 0, 16, P->ctrs + 1, P->norms_out,
+                          P->kl_sum && step == 0 ? P->kl_state : nullptr);
   CADRE_API_END
 }
 
@@ -1299,7 +1373,8 @@ int cadre_ppo_adam_step_modules(void* handle, float* params, const float* grads,
   PpoPlan* P = static_cast<PpoPlan*>(handle);
   CADRE_REQUIRE(P && params && grads && exp_avg && exp_avg_sq && step >= 0, "adam_step arguments");
   cadre::launch_clip_adam(P->opt, params, grads, exp_avg, exp_avg_sq, max_grad_norm, lr, beta1, beta2, eps, step,
-                          static_cast<cudaStream_t>(stream), mod_begin, mod_end, P->ctrs + 1, P->norms_out);
+                          static_cast<cudaStream_t>(stream), mod_begin, mod_end, P->ctrs + 1, P->norms_out,
+                          P->kl_sum && step == 0 ? P->kl_state : nullptr);
   CADRE_API_END
 }
 
@@ -1309,6 +1384,64 @@ int cadre_ppo_set_diagnostics(void* handle, float* diag_out, float* norms_out) {
   CADRE_REQUIRE(P != nullptr, "set_diagnostics: ppo handle is NULL");
   P->diag_out = diag_out;
   P->norms_out = norms_out;
+  CADRE_API_END
+}
+
+int cadre_ppo_set_target_kl(void* handle, float target_kl, int total_workers, float* kl_sum_dev) {
+  CADRE_API_BEGIN
+  CADRE_REQUIRE(std::isfinite(target_kl) && target_kl >= 0.f, "set_target_kl: target_kl must be a finite value > 0 (0: off)");
+  PpoPlan* P = static_cast<PpoPlan*>(handle);
+  CADRE_REQUIRE(P != nullptr, "set_target_kl: ppo handle is NULL");
+  if (target_kl == 0.f) {
+    P->kl_sum = nullptr;
+  } else {
+    CADRE_REQUIRE(kl_sum_dev != nullptr, "set_target_kl: kl_sum_dev is NULL");
+    CADRE_REQUIRE(total_workers >= P->cfg.workers, "set_target_kl: total_workers is below this engine's workers");
+    P->kl_limit = static_cast<float>(1.5 * static_cast<double>(target_kl));
+    P->kl_inv_total = 1.f / static_cast<float>(total_workers);
+    P->kl_sum = kl_sum_dev;
+  }
+  CADRE_API_END
+}
+
+int cadre_ppo_kl_begin(void* handle, void* stream) {
+  CADRE_API_BEGIN
+  PpoPlan* P = static_cast<PpoPlan*>(handle);
+  CADRE_REQUIRE(P != nullptr, "kl_begin: ppo handle is NULL");
+  CADRE_CUDA_CHECK(cudaMemsetAsync(P->kl_state, 0, sizeof(int) * cadre::KS_WORDS, static_cast<cudaStream_t>(stream)));
+  CADRE_API_END
+}
+
+int cadre_ppo_kl_gate(void* handle, void* stream) {
+  CADRE_API_BEGIN
+  PpoPlan* P = static_cast<PpoPlan*>(handle);
+  CADRE_REQUIRE(P != nullptr, "kl_gate: ppo handle is NULL");
+  CADRE_REQUIRE(P->kl_sum != nullptr, "kl_gate: target_kl is not set (cadre_ppo_set_target_kl)");
+  cadre::launch_k(cadre::kl_gate_kernel, dim3(1), dim3(1), 0, static_cast<cudaStream_t>(stream), P->kl_sum,
+                  P->kl_inv_total, P->kl_limit, P->kl_state, P->kl_hist, P->ctrs + 1);
+  CADRE_CUDA_CHECK(cudaGetLastError());
+  CADRE_API_END
+}
+
+int cadre_ppo_early_stop(void* handle, int32_t* state_host, float* kl_host, int kl_count, void* stream) {
+  CADRE_API_BEGIN
+  PpoPlan* P = static_cast<PpoPlan*>(handle);
+  CADRE_REQUIRE(P != nullptr && state_host != nullptr, "early_stop: NULL handle or state_host");
+  CADRE_REQUIRE(kl_count >= 0 && kl_count <= cadre::KL_HIST_CAP && (kl_count == 0 || kl_host != nullptr),
+                "early_stop: kl_count must be in [0, 4096] with kl_host set when positive");
+  // stream-ordered reads behind the phase's gates, then a wait on that stream only
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  int st[cadre::KS_WORDS], adam = 0;
+  CADRE_CUDA_CHECK(cudaMemcpyAsync(st, P->kl_state, sizeof(st), cudaMemcpyDeviceToHost, s));
+  CADRE_CUDA_CHECK(cudaMemcpyAsync(&adam, P->ctrs + 1, sizeof(int), cudaMemcpyDeviceToHost, s));
+  if (kl_count > 0)
+    CADRE_CUDA_CHECK(cudaMemcpyAsync(kl_host, P->kl_hist, sizeof(float) * kl_count, cudaMemcpyDeviceToHost, s));
+  CADRE_CUDA_CHECK(cudaStreamSynchronize(s));
+  state_host[0] = st[cadre::KS_STEP];
+  state_host[1] = st[cadre::KS_RUN];
+  state_host[2] = st[cadre::KS_APPLIED];
+  state_host[3] = st[cadre::KS_STOPPED] ? st[cadre::KS_STOPPED_AT] : -1;
+  state_host[4] = adam;
   CADRE_API_END
 }
 

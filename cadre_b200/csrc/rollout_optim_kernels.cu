@@ -215,9 +215,11 @@ __global__ void __launch_bounds__(256, (ITERS > 16 ? 3 : 1)) gae_kernel(const fl
 __global__ void __launch_bounds__(256) sqnorm_partial_kernel(const float* __restrict__ g,
                                                              const long long* __restrict__ chunk_off,
                                                              const int* __restrict__ chunk_len,
-                                                             float* __restrict__ partial) {
+                                                             float* __restrict__ partial,
+                                                             const int* __restrict__ skip) {
   pdl_trigger();
   pdl_wait();
+  if (skip && *skip) return;
   const long long off = chunk_off[blockIdx.x];
   const int len = chunk_len[blockIdx.x];
   const float4* g4 = reinterpret_cast<const float4*>(g + off);
@@ -240,9 +242,11 @@ __global__ void __launch_bounds__(256) sqnorm_partial_kernel(const float* __rest
 __global__ void sqnorm_final_kernel(const float* __restrict__ partial, const int* __restrict__ mod_first,
                                     float max_norm, float* __restrict__ clip_coef, float* __restrict__ norms,
                                     int mod_begin, int step, const int* __restrict__ dev_step, float lr, float beta1,
-                                    float beta2, float* __restrict__ scalars, float* __restrict__ norms_hist) {
+                                    float beta2, float* __restrict__ scalars, float* __restrict__ norms_hist,
+                                    const int* __restrict__ skip) {
   pdl_trigger();
   pdl_wait();
+  if (skip && *skip) return;
   // one warp per module; chunks of a module are contiguous in the chunk table
   const int m = mod_begin + blockIdx.x, lane = threadIdx.x;
   if (blockIdx.x == 0 && lane == 0) {
@@ -271,9 +275,11 @@ __global__ void __launch_bounds__(256) adam_kernel(float* __restrict__ p, const 
                                                    const int* __restrict__ chunk_len,
                                                    const int* __restrict__ chunk_mod,
                                                    const float* __restrict__ clip_coef, float beta1,
-                                                   float beta2, float eps, const float* __restrict__ scalars) {
+                                                   float beta2, float eps, const float* __restrict__ scalars,
+                                                   const int* __restrict__ skip) {
   pdl_trigger();
   pdl_wait();
+  if (skip && *skip) return;
   const float step_size = scalars[0], bc2_sqrt = scalars[1];
   const long long off = chunk_off[blockIdx.x];
   const int len = chunk_len[blockIdx.x];
@@ -302,17 +308,22 @@ __global__ void __launch_bounds__(256) adam_kernel(float* __restrict__ p, const 
 
 void launch_clip_adam(const OptTables& t, float* params, const float* grads, float* m, float* v, float max_norm,
                       float lr, float beta1, float beta2, float eps, int step, cudaStream_t s, int mod_begin,
-                      int mod_end, const int* dev_step, float* norms_hist) {
+                      int mod_end, const int* dev_step, float* norms_hist, const int* gate) {
   CADRE_REQUIRE(mod_begin >= 0 && mod_begin < mod_end && mod_end <= 16, "module range");
   CADRE_REQUIRE(step >= 1 || dev_step != nullptr, "Adam step");
   // chunks of modules [mod_begin, mod_end) are contiguous in the chunk table (it is sorted by module)
   const int c0 = t.mod_first_h[mod_begin], nc = t.mod_first_h[mod_end] - c0;
   if (nc <= 0) return;
-  launch_k(sqnorm_partial_kernel, dim3(nc), dim3(256), 0, s, grads, t.chunk_off + c0, t.chunk_len + c0, t.partial + c0);
+  // gate: the target-KL state words (ppo.cu, kl_gate_kernel): [0] the phase stopped before this step (no norms either),
+  // [1] the phase is stopped (no Adam update)
+  const int* skip_norm = gate;
+  const int* skip_adam = gate ? gate + 1 : nullptr;
+  launch_k(sqnorm_partial_kernel, dim3(nc), dim3(256), 0, s, grads, t.chunk_off + c0, t.chunk_len + c0, t.partial + c0,
+           skip_norm);
   launch_k(sqnorm_final_kernel, dim3(mod_end - mod_begin), dim3(32), 0, s, t.partial, t.mod_first, max_norm, t.clip_coef,
-           t.norms, mod_begin, step, dev_step, lr, beta1, beta2, t.scalars, norms_hist);
+           t.norms, mod_begin, step, dev_step, lr, beta1, beta2, t.scalars, norms_hist, skip_norm);
   launch_k(adam_kernel, dim3(nc), dim3(256), 0, s, params, grads, m, v, t.chunk_off + c0, t.chunk_len + c0, t.chunk_mod + c0,
-           t.clip_coef, beta1, beta2, eps, t.scalars);
+           t.clip_coef, beta1, beta2, eps, t.scalars, skip_adam);
   CADRE_CUDA_CHECK(cudaGetLastError());
 }
 

@@ -12,6 +12,8 @@ replicas hold identical parameters afterwards. How it is done here:
     (agent.py:239-243) is needed and replicas stay bit-identical.
 """
 import ctypes
+import math
+import numbers
 import os
 
 import numpy as np
@@ -22,6 +24,19 @@ from . import ppo as _ppo
 from ._lib import CadreError
 from . import ppo_params
 from .storage import RolloutStorage
+
+KL_TAIL = 4              # floats past the gradient that carry the per-head KL sums through the gradient exchange
+KL_HIST_STEPS = 4096     # update steps of one learn() phase the engine keeps the KL of (csrc/ppo.cu, KL_HIST_CAP)
+
+
+def check_target_kl(target_kl):
+    """None (early stopping off) or a finite float > 0 that stays finite and > 0 in float32; raises CadreError."""
+    if target_kl is None:
+        return None
+    v = float(target_kl) if isinstance(target_kl, numbers.Real) and not isinstance(target_kl, bool) else math.nan
+    if not (math.isfinite(v) and v <= float(np.finfo(np.float32).max) and np.float32(v) > 0):
+        raise CadreError(f"target_kl={target_kl!r}: expected None (off) or a finite float > 0")
+    return v
 
 
 class RolloutPool:
@@ -107,9 +122,15 @@ class RolloutPool:
 
 class Learner:
     def __init__(self, workers, mini_batch, ppo_state, device="cuda:0", clip=0.1, value_coeff=0.1, clip_coeff=1.0,
-                 ent_coeff=0.01, lr=3e-4, max_grad_norm=250.0, process_group=None, seeds=None, diagnostics=False):
+                 ent_coeff=0.01, lr=3e-4, max_grad_norm=250.0, process_group=None, seeds=None, diagnostics=False,
+                 target_kl=None):
         """`diagnostics`: record, for every update step, the approximate KL, clip fractions and pre-clip module gradient
-        norms in device-side histories (no host synchronisation inside a phase); read them with `diagnostics()`."""
+        norms in device-side histories (no host synchronisation inside a phase); read them with `diagnostics()`.
+        `target_kl` (None: off): early stopping of each `learn()` phase by SB3's rule. The KL of update step n is the sum
+        over the two heads of the mean over all workers of all ranks of the approximate KL; when it exceeds
+        1.5 * target_kl, step n is not applied and the phase's later steps are skipped, decided on the device with the
+        same bits on every rank. `early_stop()` reports the outcome."""
+        target_kl = check_target_kl(target_kl)
         self.device = torch.device(device)
         self.workers, self.mini_batch = workers, mini_batch
         self.value_coeff, self.clip_coeff, self.ent_coeff = value_coeff, clip_coeff, ent_coeff
@@ -119,6 +140,10 @@ class Learner:
         self.world = 1
         if process_group is not None or (torch.distributed.is_available() and torch.distributed.is_initialized()):
             self.world = torch.distributed.get_world_size(process_group)
+        self.target_kl = target_kl
+        # with target_kl the gradient buffer has a KL_TAIL-float tail past the parameters (the Adam chunk table never
+        # reaches it): head_kernel writes this rank's per-head KL sums there, and the gradient exchange sums them
+        n_grad = self.params.numel() + (KL_TAIL if target_kl is not None else 0)
         # Gradient exchange: "switch" = the library's in-switch reduction on a symmetric gradient buffer
         # (collective.SwitchAllReduce, csrc/allreduce.cu), "nccl" = torch.distributed.all_reduce. "auto" (default) takes
         # the switch from 4 ranks on when the fabric offers a multicast mapping: measured on 8 x B200 the 77.9 MB sum
@@ -131,7 +156,7 @@ class Learner:
         if self.exchange == "switch" or (self.exchange == "auto" and self.world >= 4):
             from .collective import SwitchAllReduce
             try:
-                self._switch = SwitchAllReduce(self.params.numel(), self.device, process_group)
+                self._switch = SwitchAllReduce(n_grad, self.device, process_group)
             except Exception as e:     # no symmetric memory between these devices (not one NVLink domain, two ranks per GPU)
                 if self.exchange == "switch":
                     raise
@@ -141,18 +166,27 @@ class Learner:
                 self._switch = None    # peer loads / stores only pay off between two GPUs
         if self._switch is not None:
             self.exchange = "switch"
-            self.grads = self._switch.buffer
+            self._grad_buf = self._switch.buffer
         else:
             self.exchange = "nccl" if self.world > 1 else "none"
-            self.grads = torch.zeros_like(self.params)
+            self._grad_buf = torch.zeros(n_grad, dtype=self.params.dtype, device=self.device)
+        self.grads = self._grad_buf if target_kl is None else self._grad_buf[:self.params.numel()]
+        if target_kl is not None:
+            self.engine.set_target_kl(target_kl, workers * self.world, self._grad_buf[self.params.numel():])
         self.exp_avg = torch.zeros_like(self.params)
         self.exp_avg_sq = torch.zeros_like(self.params)
         self.losses = torch.zeros(workers, 2, 3, device=self.device)       # last update step
         self.loss_sum = torch.zeros(workers, 2, 3, device=self.device)     # summed over the update steps of learn()
         self.loss_steps = 0
-        self.step_count = 0
+        self._step_count = 0
         self.diagnostics_on = bool(diagnostics)
         self._diag_hist = self._norm_hist = None      # [steps, W, 2, 4] and [steps, 16] of the last learn() / update_step
+        self._diag_of_learn = False
+        # target_kl: the last learn() phase while its outcome is on the device only (_resolve_phase reads it), its
+        # per-step losses [steps, W, 2, 3], and the outcome once read
+        self._phase = None
+        self._loss_hist = None
+        self._early_stop = None
         self.pg = process_group
         self.overlap_allreduce = os.environ.get("CADRE_NO_ALLREDUCE_OVERLAP", "0") != "1"
         self._comm_stream = None
@@ -214,8 +248,20 @@ class Learner:
         assert lstm[-1][0] + lstm[-1][1] == mlp[0] and lstm[-1][3] == mlp[2]      # contiguous ranges and module ids
         self._ranges = lstm[:-1] + [(lstm[-1][0], lstm[-1][1] + mlp[1], lstm[-1][2], mlp[3])]
         self._waits = [[g] for g in range(groups - 1)] + [[groups - 1, -1]]
+        self._kl_tail = None
+        if self.target_kl is not None:
+            # the KL sums must be summed before range 0 is stepped: in the one range when there is one, else by a
+            # 16-byte exchange of their own issued before range 0's (after the BPTT kernel, like every collective here)
+            if len(self._ranges) == 1:
+                # (an exchange with no gated step before it - update_step, a skipped step - sums the stale tail again;
+                # after a sum every rank holds the same values, so repeats only scale them, at worst to +-inf and never
+                # to NaN, and the gate reads the tail only after head_kernel has rewritten it)
+                off, cnt, m0, m1 = self._ranges[0]
+                self._ranges[0] = (off, cnt + KL_TAIL, m0, m1)
+            else:
+                self._kl_tail = (self.params.numel(), KL_TAIL)
         self._reduced = [torch.cuda.Event() for _ in self._ranges]
-        assert sum(r[1] for r in self._ranges) == self.grads.numel()
+        assert sum(r[1] for r in self._ranges) + (KL_TAIL if self._kl_tail else 0) == self._grad_buf.numel()
         assert all(r[0] % 4 == 0 and r[1] % 4 == 0 for r in self._ranges)        # 16-byte vectors in the exchange
 
     def _exchange_and_step(self, step):
@@ -227,46 +273,63 @@ class Learner:
         flat buffer; a communication stream all-reduces range k as soon as its event fires while the GEMMs of group
         k+1 still run, and the main stream applies clip + Adam to the modules of range k - a per-module operation,
         chief.py:16-21 - while range k+1 is on the wire. Sums, clip coefficients and Adam arithmetic are those of the
-        single all-reduce + single step."""
+        single all-reduce + single step.
+        With target_kl, a staged step (step = 0) is gated after the KL sums have been summed across ranks and before
+        the first clip + Adam of the step."""
+        gate = self.target_kl is not None and step == 0
         if self.world > 1:
             main = torch.cuda.current_stream(self.device)
             with torch.cuda.stream(self._comm_stream):
                 for k, (off, cnt, _, _) in enumerate(self._ranges):
                     for g in self._waits[k]:
                         self.engine.wait_grads(g, self._comm_stream)
-                    if self._switch is not None:
-                        self._switch.sum_(off, cnt, stream=self._comm_stream)
-                    else:
-                        torch.distributed.all_reduce(self.grads[off:off + cnt], op=torch.distributed.ReduceOp.SUM,
-                                                     group=self.pg)
+                    if k == 0 and gate and self._kl_tail is not None:
+                        self._sum_over_ranks(*self._kl_tail)
+                    self._sum_over_ranks(off, cnt)
                     self._reduced[k].record(self._comm_stream)
             for k, (_, _, m0, m1) in enumerate(self._ranges):
                 main.wait_event(self._reduced[k])
+                if k == 0 and gate:
+                    self.engine.kl_gate()
                 self.engine.adam_step_modules(self.params, self.grads, self.exp_avg, self.exp_avg_sq, step, m0, m1,
                                               self.max_grad_norm, self.lr)
         else:
+            if gate:
+                self.engine.kl_gate()
             self.engine.adam_step(self.params, self.grads, self.exp_avg, self.exp_avg_sq, step, self.max_grad_norm,
                                   self.lr)
-        self.loss_sum += self.losses
-        self.loss_steps += 1
+        if not gate:        # (a gated phase keeps per-step losses instead: _resolve_phase)
+            self.loss_sum += self.losses
+            self.loss_steps += 1
+
+    def _sum_over_ranks(self, off, cnt):
+        """[off, off + cnt) of the gradient buffer <- its sum over ranks, on the current (communication) stream."""
+        if self._switch is not None:
+            self._switch.sum_(off, cnt, stream=self._comm_stream)
+        else:
+            torch.distributed.all_reduce(self._grad_buf[off:off + cnt], op=torch.distributed.ReduceOp.SUM, group=self.pg)
 
     def update_step(self, storages, indices, async_losses=True):
         """update_policy for all local workers -> all-reduce(sum) -> per-module clip + Adam (one step, eagerly).
         storages[w] = (steer, throttle) RolloutStorage with `.advantages`; indices int32 [W,2,mb]."""
         advs = [(s.advantages, t.advantages) for s, t in storages]
+        self._resolve_phase()      # (after a gated learn(): the Adam step actually reached)
         if self.world > 1 and self._comm_stream is None:
             self._setup_pipeline()
+        self._diag_of_learn = False
         self._diag_step(0, 1)
         self.engine.update(storages, advs, indices, self.params, self.grads, self.losses)
-        self.step_count += 1
-        self._exchange_and_step(self.step_count)
+        self._step_count += 1
+        self._exchange_and_step(self._step_count)
         self._diag_step(None)
         return self.losses if async_losses else self.scaled_losses()
 
     def scaled_losses(self, mean=False):
         """[W,3] = (value_loss*coeff, action_loss*coeff, entropy*coeff) per worker, like update_policy's return:
         of the LAST update step, or with `mean=True` averaged over the update steps since the last `learn()` began
-        (what train.py:98-100, 112-116 logs)."""
+        (what train.py:98-100, 112-116 logs). After a learn() stopped by target_kl: of the steps that ran their
+        forward (the applied ones and the one that stopped the phase)."""
+        self._resolve_phase()
         L = (self.loss_sum / max(1, self.loss_steps) if mean else self.losses).sum(1).cpu()
         return L * torch.tensor([self.value_coeff, self.clip_coeff, self.ent_coeff])
 
@@ -284,19 +347,74 @@ class Learner:
             self._setup_pipeline()
         idx_all = np.concatenate([self.sample_epoch_indices(storages) for _ in range(ppo_epoch)], 0)
         advs = [(s.advantages, t.advantages) for s, t in storages]
+        steps = idx_all.shape[0]
+        gate = self.target_kl is not None
+        if gate:
+            if steps > KL_HIST_STEPS:
+                raise CadreError(f"learn(): {steps} update steps in one phase; target_kl supports up to {KL_HIST_STEPS}")
+            # the Adam step of the first staged step: the host's count, or, while the previous gated phase is unread,
+            # the device counter it left (the steps it actually applied)
+            first = 0 if self._phase is not None else self._step_count + 1
+            self._loss_hist = torch.zeros(steps, self.workers, 2, 3, device=self.device)
+            self._phase, self._early_stop = dict(steps=steps), None
+            self.engine.kl_begin()
+        self._diag_of_learn = True
         n = 0
-        while n < idx_all.shape[0]:                       # (the staging table holds 64 steps)
-            m = min(64, idx_all.shape[0] - n)
-            self.engine.stage(storages, advs, idx_all[n:n + m], self.step_count + 1)
+        while n < steps:                                  # (the staging table holds 64 steps)
+            m = min(64, steps - n)
+            self.engine.stage(storages, advs, idx_all[n:n + m], (first if n == 0 else 0) if gate else self._step_count + 1)
             for k in range(m):
-                self._diag_step(n + k, idx_all.shape[0])
-                self.engine.update_staged(self.params, self.grads, self.losses)
+                self._diag_step(n + k, steps)
+                self.engine.update_staged(self.params, self.grads, self._loss_hist[n + k] if gate else self.losses)
                 self._exchange_and_step(0)
-                self.step_count += 1
+                if not gate:
+                    self._step_count += 1
             n += m
         self._diag_step(None)
-        self.loss_steps = idx_all.shape[0]
-        return idx_all.shape[0]
+        self.loss_steps = steps
+        return steps
+
+    @property
+    def step_count(self):
+        """Adam steps applied so far (after a gated learn(), reading it synchronises once). Callers that step the
+        optimizer themselves (utils.chief) may assign it, as with a plain attribute."""
+        self._resolve_phase()
+        return self._step_count
+
+    @step_count.setter
+    def step_count(self, value):
+        self._resolve_phase()
+        self._step_count = value
+
+    def _resolve_phase(self):
+        """After a learn() with target_kl: read its outcome (one synchronisation) into the Adam step count, the losses
+        of the last step that ran and their sum over the steps that ran. Nothing to do otherwise."""
+        if self._phase is None:
+            return
+        steps = self._phase["steps"]
+        r = self.engine.early_stop(steps)
+        kl = r["kl"]
+        kl[r["run"]:] = np.nan
+        self._early_stop = dict(steps=steps, applied=r["applied"], stopped_at=r["stopped_at"], kl=kl)
+        self._step_count = r["adam_step"]
+        self.loss_sum.zero_()
+        for i in range(r["run"]):                         # the same sum, in the same order, as an ungated phase
+            self.loss_sum += self._loss_hist[i]
+        self.losses.copy_(self._loss_hist[r["run"] - 1])
+        self.loss_steps = r["run"]
+        self._phase = None
+
+    def early_stop(self):
+        """Outcome of the last learn() with target_kl (one synchronisation): {"steps": staged steps, "applied": steps
+        whose Adam update was applied, "stopped_at": index of the step whose KL exceeded 1.5 * target_kl (it was not
+        applied, nor were the steps after it) or None, "kl": float32 [steps] KL of each step, NaN for steps that did not
+        run}."""
+        if self.target_kl is None:
+            raise CadreError("early_stop() needs Learner(..., target_kl=...)")
+        self._resolve_phase()
+        if self._early_stop is None:
+            raise CadreError("early_stop(): no learn() phase has run yet")
+        return dict(self._early_stop, kl=self._early_stop["kl"].copy())
 
     # ---------------------------------------------------------------- diagnostics
     def _diag_step(self, k, steps=None):
@@ -307,9 +425,10 @@ class Learner:
         if k is None:
             self.engine.set_diagnostics(None, None)
             return
-        if k == 0:
-            self._diag_hist = torch.zeros(steps, self.workers, 2, len(_ppo.DIAG_TERMS), device=self.device)
-            self._norm_hist = torch.zeros(steps, 16, device=self.device)
+        if k == 0:    # (with target_kl, rows of steps that do not run stay NaN)
+            fill = math.nan if self.target_kl is not None else 0.0
+            self._diag_hist = torch.full((steps, self.workers, 2, len(_ppo.DIAG_TERMS)), fill, device=self.device)
+            self._norm_hist = torch.full((steps, 16), fill, device=self.device)
         self.engine.set_diagnostics(self._diag_hist[k], self._norm_hist[k])
 
     def diagnostics(self):
@@ -318,7 +437,9 @@ class Learner:
         `kl_k1` (mean of -d), `clip_frac` (rows with |ratio - 1| > clip) and `value_clip_frac` (rows with
         |value - old value| > clip); [steps, 16]: `grad_norm`, every module's gradient norm before clipping (after the
         all-reduce, so the same on every rank), columns in `modules` order (the reference's model_dict order), and
-        `grad_clipped` = grad_norm > max_grad_norm."""
+        `grad_clipped` = grad_norm > max_grad_norm.
+        With target_kl also `applied`, bool [steps], and `stopped_at` (see `early_stop()`); rows of steps that did not
+        run are NaN, the row of the step that stopped the phase holds its values."""
         if not self.diagnostics_on:
             raise CadreError("diagnostics() needs Learner(..., diagnostics=True)")
         if self._diag_hist is None:
@@ -334,6 +455,13 @@ class Learner:
         out["grad_norm"] = norms[:, cols]
         out["grad_clipped"] = out["grad_norm"] > self.max_grad_norm
         out["modules"] = modules
+        if self.target_kl is not None:
+            if self._diag_of_learn:
+                es = self.early_stop()
+                out["applied"] = np.arange(steps) < es["applied"]
+                out["stopped_at"] = es["stopped_at"]
+            else:
+                out["applied"], out["stopped_at"] = np.ones(steps, dtype=bool), None
         return out
 
     def check(self):

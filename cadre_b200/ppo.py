@@ -105,7 +105,7 @@ class PpoEngine:
     def stage(self, storages, advantages, indices_all, first_adam_step):
         """Upload the storage references and the indices of a SEQUENCE of update steps, int [n_steps, W, 2, mb]; each
         following `update_staged` consumes the next slice and advances the device-side Adam step (the first one is
-        `first_adam_step`, 1-based), which `adam_step*` use when called with step=0."""
+        `first_adam_step`, 1-based; 0 continues the device counter), which `adam_step*` use when called with step=0."""
         assert len(storages) == self.workers and len(advantages) == self.workers
         for w in range(self.workers):
             for h in range(2):
@@ -213,6 +213,42 @@ class PpoEngine:
                     raise _lib.CadreError(f"set_diagnostics: `{name}` must hold {n} floats on {self.device} "
                                           f"(got {t.numel()} on {t.device})")
         _lib.check(self._lib.cadre_ppo_set_diagnostics(self._h, _lib.ptr(diag), _lib.ptr(norms)))
+
+    def set_target_kl(self, target_kl, total_workers=None, kl_sum=None):
+        """Target-KL early stopping of staged phases (cadre_ppo_set_target_kl): None or 0 turns it off; otherwise
+        `total_workers` is the worker count of all ranks and `kl_sum` fp32 [4] on this device receives each staged
+        update's per-head KL sums in [0:2] (sum it over ranks, then `kl_gate`). It must stay alive while it is set."""
+        if target_kl is None or target_kl == 0:
+            _lib.check(self._lib.cadre_ppo_set_target_kl(self._h, ctypes.c_float(0.0), 0, None))
+            return
+        if kl_sum is not None:
+            _check_tensor(kl_sum, torch.float32, "kl_sum")
+            if kl_sum.numel() < 2:
+                raise _lib.CadreError(f"set_target_kl: `kl_sum` must hold at least 2 floats (got {kl_sum.numel()})")
+        _lib.check(self._lib.cadre_ppo_set_target_kl(
+            self._h, ctypes.c_float(target_kl), int(total_workers if total_workers is not None else self.workers),
+            _lib.ptr(kl_sum)))
+
+    def kl_begin(self):
+        """Start a phase of staged steps: clear the early stop (cadre_ppo_kl_begin)."""
+        with torch.cuda.device(self.device):
+            _lib.check(self._lib.cadre_ppo_kl_begin(self._h, _lib.stream_ptr(self.device)))
+
+    def kl_gate(self):
+        """The stop decision of the current staged step (cadre_ppo_kl_gate), after the cross-rank sum of `kl_sum`."""
+        with torch.cuda.device(self.device):
+            _lib.check(self._lib.cadre_ppo_kl_gate(self._h, _lib.stream_ptr(self.device)))
+
+    def early_stop(self, kl_count=0):
+        """Wait for the current stream and read the phase's early-stop state (cadre_ppo_early_stop): dict with `gated`, `run`,
+        `applied`, `stopped_at` (None: no stop), `adam_step` (the device Adam step) and `kl` float32 [kl_count]."""
+        st = (ctypes.c_int32 * 5)()
+        kl = np.zeros(int(kl_count), dtype=np.float32)
+        with torch.cuda.device(self.device):
+            _lib.check(self._lib.cadre_ppo_early_stop(self._h, st, kl.ctypes.data_as(ctypes.c_void_p) if kl_count else None,
+                                                      int(kl_count), _lib.stream_ptr(self.device)))
+        return dict(gated=st[0], run=st[1], applied=st[2], stopped_at=None if st[3] < 0 else st[3], adam_step=st[4],
+                    kl=kl)
 
     def check(self):
         """Synchronise and raise CadreError if a recurrence kernel of an earlier call timed out on a hand-off."""

@@ -27,7 +27,9 @@ def train(rank, train_cfg, agent_cfg, env_cfg, rollout_cfg, danet_state, ppo_sta
     path's.
     `diagnostics` records the PPO update diagnostics of every episode (`Learner.diagnostics`, `RolloutPool.rollout_stats`):
     each `history` entry gains a dict of them as a fourth element, and rank 0 logs one more line per `log_interval`.
-    Values are those of this rank's workers. Training itself is unchanged."""
+    Values are those of this rank's workers. Training itself is unchanged.
+    `train_cfg.target_kl` (absent or None: off) stops each PPO phase early by SB3's rule (`Learner(target_kl=...)`);
+    rank 0 logs one more line per `log_interval` when the phase stopped."""
     if device_rollout and not batched_acting:
         raise ValueError("device_rollout=True needs batched_acting=True")
     device = torch.device("cuda:" + str(agent_cfg.model_cfg.device_num))
@@ -41,7 +43,7 @@ def train(rank, train_cfg, agent_cfg, env_cfg, rollout_cfg, danet_state, ppo_sta
     learner = Learner(workers, mb, ppo_state, device, agent_cfg.clip, agent_cfg.value_coeff, agent_cfg.clip_coeff,
                       agent_cfg.ent_coeff, train_cfg.lr, train_cfg.max_grad_norm, process_group,
                       seeds=[env_cfg.get("seed", 0) + rank * workers + w for w in range(workers)],
-                      diagnostics=diagnostics)
+                      diagnostics=diagnostics, target_kl=train_cfg.get("target_kl"))
     agent.owner.params = learner.params          # the acting replica reads the learner's parameters directly
     pool = RolloutPool(workers, dict(rollout_cfg, hidden_size=hidden_size), device)
     obs = [e.reset() for e in envs]
@@ -86,6 +88,11 @@ def train(rank, train_cfg, agent_cfg, env_cfg, rollout_cfg, danet_state, ppo_sta
             log("Episode: {}, value loss: {:.4f}, policy loss: {:.4f}, entropy loss: {:.4f}".format(episode, *L))
             if diagnostics:
                 log(_diagnostics_line(episode, diag))
+            if learner.target_kl is not None:
+                es = learner.early_stop()
+                if es["stopped_at"] is not None:
+                    log("Episode: {}, early stop at update step {} of {} (kl {:.1e} > 1.5 x {:.1e})".format(
+                        episode, es["stopped_at"], es["steps"], es["kl"][es["stopped_at"]], learner.target_kl))
     return learner, history
 
 

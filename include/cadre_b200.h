@@ -254,6 +254,25 @@ int cadre_ppo_launches(void* handle);
  * device-side history before each staged step, which needs no synchronisation. NULL turns either off; losses,
  * gradients and parameters do not depend on the setting. */
 int cadre_ppo_set_diagnostics(void* handle, float* diag_out, float* norms_out);
+/* Target-KL early stopping of a phase of staged update steps (off by default; SB3's target_kl rule). While it is on,
+ * each staged cadre_ppo_update also writes kl_sum_dev fp32 [2]: per head, the sum over this engine's workers of the
+ * approximate KL (diag term [0] above). The caller sums kl_sum_dev over ranks (a 16-byte vector in place) and then
+ * calls cadre_ppo_kl_gate on the stream of the Adam steps, before the step's first cadre_ppo_adam_step* with step = 0.
+ * The gate computes KL = sum over heads of kl_sum[h] * (1 / total_workers); if KL > 1.5 * target_kl the step is not
+ * applied (no norms are skipped for it, but no Adam update, no moment update, and the device Adam step goes back by
+ * one), and every later step of the phase is skipped: its update routes no rows (gradients and losses are zeros) and its
+ * norms and Adam step do nothing. One-step updates (indices_host set) and Adam steps with step >= 1 ignore the gate.
+ * cadre_ppo_set_target_kl: target_kl = 0 turns it off; otherwise target_kl must be finite and > 0, total_workers (all
+ * ranks) >= this engine's workers and kl_sum_dev set (4 floats advised: a 16-byte vector for the exchange).
+ * cadre_ppo_kl_begin starts a phase (clears the stop); call it before the phase's first cadre_ppo_stage, not between
+ * its chunks. cadre_ppo_stage with first_adam_step = 0 continues the device Adam step (after a stop, the steps actually
+ * applied). cadre_ppo_early_stop reads the state in the order of `stream` (the stream of the gates), waits for that
+ * stream only, and returns state_host int32 [5] = steps gated, steps run (applied + the one that stopped), steps applied, index of the step that stopped (-1: none), device Adam step; and kl_host fp32
+ * [kl_count] (kl_count <= 4096), the KL of each step that ran (entries past "steps run" are stale). */
+int cadre_ppo_set_target_kl(void* handle, float target_kl, int total_workers, float* kl_sum_dev);
+int cadre_ppo_kl_begin(void* handle, void* stream);
+int cadre_ppo_kl_gate(void* handle, void* stream);
+int cadre_ppo_early_stop(void* handle, int32_t* state_host, float* kl_host, int kl_count, void* stream);
 
 /* ------------------------------------------------------------------------------------------------------
  * Device-side rollout collection: replaces the host-side Categorical draw (ppo_agent/distributions.py:96-99,
