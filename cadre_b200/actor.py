@@ -110,6 +110,25 @@ class BatchedActor:
         """Forget environment `env_id`'s window (call after env.reset())."""
         self._last[env_id] = None
 
+    # ------------------------------------------------------------------ checkpoints
+    def state_dict(self):
+        """What the next tick depends on: the sampler's counter (`ticks`, `seed`, `env_ids`), the frame cache (`feats`
+        on the host, `_last`, whose arrays are private copies that are replaced, never modified) and `frames_encoded`."""
+        return dict(ticks=self.ticks, seed=self.seed, env_ids=list(self.env_ids), feats=self.feats.cpu(),
+                    last=list(self._last),
+                    frames_encoded=self.frames_encoded)
+
+    def load_state_dict(self, state):
+        """Restore a `state_dict()` of an actor with the same number of environments (`feats` in place: the forward's
+        storage views read it)."""
+        if len(state["env_ids"]) != self.E or tuple(state["feats"].shape) != tuple(self.feats.shape):
+            raise ValueError(f"actor state of {len(state['env_ids'])} environments, this actor steps {self.E}")
+        self.ticks, self.seed, self.frames_encoded = int(state["ticks"]), int(state["seed"]), int(state["frames_encoded"])
+        self.env_ids = [int(i) for i in state["env_ids"]]
+        self._env_ids_d.copy_(torch.tensor(self.env_ids, dtype=torch.int32))
+        self.feats.copy_(state["feats"])
+        self._last = list(state["last"])
+
     # ------------------------------------------------------------------ acting
     def act_batch(self, ticks):
         """One tick of all E environments. Returns (features [E,8,530], actions int64 [E,2], log_probs [E,2],

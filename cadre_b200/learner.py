@@ -119,6 +119,26 @@ class RolloutPool:
         out = _ppo.rollout_stats(b["returns"].view(n, T + 1), b["value_preds"].view(n, T + 1)).cpu().numpy()
         return {name: out[:, k].reshape(self.workers, 2) for k, name in enumerate(_ppo.ROLLOUT_STATS)}
 
+    def state_dict(self):
+        """Host copies of the batched tensors and `next_value`, and every storage's `step` cursor ([W][2]). The cursor is
+        never reset (storage.py quirk 4), so the next rollout and its GAE read the slot the last one left."""
+        return dict(batched={k: t.cpu() for k, t in self.batched.items()}, next_value=self.next_value.cpu(),
+                    steps=[[st.step for st in pair] for pair in self.storages])
+
+    def load_state_dict(self, state):
+        """Restore a `state_dict()` in place (the storages are views of the batched tensors, and `c_ref` holds their
+        addresses)."""
+        for k, t in self.batched.items():
+            if k not in state["batched"] or state["batched"][k].shape != t.shape:
+                raise CadreError(f"RolloutPool.load_state_dict: tensor {k!r} missing or of another shape")
+            t.copy_(state["batched"][k])
+        self.next_value.copy_(state["next_value"])
+        if len(state["steps"]) != self.workers:
+            raise CadreError(f"RolloutPool.load_state_dict: {len(state['steps'])} workers in the state, {self.workers} here")
+        for pair, steps in zip(self.storages, state["steps"]):
+            for st, s in zip(pair, steps):
+                st.step = int(s)
+
 
 class Learner:
     def __init__(self, workers, mini_batch, ppo_state, device="cuda:0", clip=0.1, value_coeff=0.1, clip_coeff=1.0,
@@ -473,3 +493,29 @@ class Learner:
 
     def state(self):
         return ppo_params.unpack_state(self.params)
+
+    # ---------------------------------------------------------------- checkpoints
+    def state_dict(self):
+        """Host copies of the optimizer state: params, exp_avg, exp_avg_sq, the Adam step count (after a gated learn(),
+        the steps actually applied: one synchronisation), the parameter count of the library and the per-worker
+        minibatch RNG states."""
+        self._resolve_phase()
+        return dict(params=self.params.cpu(), exp_avg=self.exp_avg.cpu(), exp_avg_sq=self.exp_avg_sq.cpu(),
+                    step_count=self._step_count, param_count=int(_lib.lib().cadre_ppo_param_count()),
+                    rng_states=[s.clone() for s in self._rng_states])
+
+    def load_state_dict(self, state):
+        """Restore a `state_dict()`. params and the moments are copied in place: the acting replica
+        (`agent.owner.params`) aliases `params`, and the gradient buffer may be symmetric memory, so no tensor is
+        rebound. The next learn() takes its first Adam step from the restored count."""
+        n = self.params.numel()
+        if int(state["param_count"]) != n or any(state[k].numel() != n for k in ("params", "exp_avg", "exp_avg_sq")):
+            raise CadreError(f"load_state_dict: {state['param_count']} parameters in the state, the learner has {n}")
+        if len(state["rng_states"]) != len(self._rng_states):
+            raise CadreError(f"load_state_dict: {len(state['rng_states'])} minibatch RNG streams in the state, the "
+                             f"learner has {len(self._rng_states)}")
+        for k in ("params", "exp_avg", "exp_avg_sq"):
+            getattr(self, k).copy_(state[k].reshape(-1))
+        self._step_count = int(state["step_count"])
+        self._rng_states = [s.clone() for s in state["rng_states"]]
+        self._phase = self._early_stop = None

@@ -36,6 +36,15 @@ class SyntheticEnv:
         self._hist = [first for _ in range(self.seq)]   # env_wrapper.py:680-688: history primed with frame 0
         return self._tick()
 
+    def get_state(self):
+        """What the next tick depends on: the generator state and the frame history (its frames are never modified in
+        place, so the list is not copied)."""
+        return {"rng": self.rs.get_state(), "hist": None if self._hist is None else list(self._hist)}
+
+    def set_state(self, state):
+        self.rs.set_state(state["rng"])
+        self._hist = None if state["hist"] is None else list(state["hist"])
+
     def step(self, output_action):
         self._hist = self._hist[1:] + [self._frame()]
         reward = torch.tensor(self.rs.rand(2).astype(np.float32))

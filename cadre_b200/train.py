@@ -7,16 +7,19 @@ import os
 import numpy as np
 import torch
 
+from . import checkpoint
 from .actor import BatchedActor
 from .agent import CadreAgent
 from .config import load_config
+from .eval import snapshot_path
 from .learner import Learner, RolloutPool
 from .models import get_vae_output, init_state
 from .synthetic_env import SyntheticEnv
 
 
 def train(rank, train_cfg, agent_cfg, env_cfg, rollout_cfg, danet_state, ppo_state=None, workers=1, max_episode=None,
-          process_group=None, log=print, batched_acting=True, device_rollout=False, diagnostics=False):
+          process_group=None, log=print, batched_acting=True, device_rollout=False, diagnostics=False,
+          checkpoint_dir=None, resume=None):
     """One rank: `workers` logical workers (env + rollout pair each) sharing one agent replica. With
     `batched_acting` the rank's workers are stepped together through `BatchedActor` (one encoder batch of the newest
     frames + one routed LSTM / head evaluation per tick) instead of one `agent.act` call per worker.
@@ -29,7 +32,15 @@ def train(rank, train_cfg, agent_cfg, env_cfg, rollout_cfg, danet_state, ppo_sta
     each `history` entry gains a dict of them as a fourth element, and rank 0 logs one more line per `log_interval`.
     Values are those of this rank's workers. Training itself is unchanged.
     `train_cfg.target_kl` (absent or None: off) stops each PPO phase early by SB3's rule (`Learner(target_kl=...)`);
-    rank 0 logs one more line per `log_interval` when the phase stopped."""
+    rank 0 logs one more line per `log_interval` when the phase stopped.
+    `checkpoint_dir` (None: no file is written): rank 0 writes the reference's snapshot
+    `<checkpoint_dir>/models/ppo_model_<episode>.pt` after every episode with episode % save_interval == 0
+    (train.py:121-123), and at those points and after the last episode every rank takes part in a training checkpoint
+    `<checkpoint_dir>/ep_<episodes completed>` (`cadre_b200.checkpoint`). `resume`: "latest" (the newest complete
+    checkpoint under `checkpoint_dir`; none yet: start from episode 0) or an ep_<n> directory. The resumed run continues
+    the same trajectory bit for bit, needs the same structural config (world size, workers per rank, shapes, env seed,
+    acting path, encoder weights) and takes the hyperparameters from the current config. `max_episode` counts all
+    episodes of the run, and the returned `history` includes the restored entries."""
     if device_rollout and not batched_acting:
         raise ValueError("device_rollout=True needs batched_acting=True")
     device = torch.device("cuda:" + str(agent_cfg.model_cfg.device_num))
@@ -54,7 +65,23 @@ def train(rank, train_cfg, agent_cfg, env_cfg, rollout_cfg, danet_state, ppo_sta
                              env_ids=[rank * workers + w for w in range(workers)])
     else:
         actor = BatchedActor(agent, workers) if batched_acting else None
-    for episode in range(max_episode if max_episode is not None else train_cfg.max_episode):
+    total = max_episode if max_episode is not None else train_cfg.max_episode
+    start = 0
+    if checkpoint_dir is not None or resume is not None:
+        ckpt_cfg = checkpoint.run_config(learner.world, workers, train_cfg, agent_cfg, env_cfg, rollout_cfg, hidden_size,
+                                         learner.params.numel(), batched_acting, device_rollout,
+                                         checkpoint.encoder_fingerprint(danet_state))
+    if resume is not None:
+        path = checkpoint.resolve(resume, checkpoint_dir)
+        if path is None:
+            if rank == 0:
+                log(f"Resume: no complete checkpoint under {checkpoint_dir}, starting from episode 0")
+        else:
+            start, history = _restore(path, rank, ckpt_cfg, learner, pool, actor, envs, obs, done, device,
+                                      log if rank == 0 else None)
+            if rank == 0:
+                log(f"Resume: {path}, {start} episodes done")
+    for episode in range(start, total):
         if device_rollout:
             _device_rollout(actor, agent, envs, pool, obs, done, num_steps)
             actor.bootstrap_into(pool, done)                              # train.py:76-79, into pool.next_value
@@ -93,7 +120,37 @@ def train(rank, train_cfg, agent_cfg, env_cfg, rollout_cfg, danet_state, ppo_sta
                 if es["stopped_at"] is not None:
                     log("Episode: {}, early stop at update step {} of {} (kl {:.1e} > 1.5 x {:.1e})".format(
                         episode, es["stopped_at"], es["steps"], es["kl"][es["stopped_at"]], learner.target_kl))
+        if checkpoint_dir is not None and (episode % train_cfg.save_interval == 0 or episode == total - 1):
+            if rank == 0 and episode % train_cfg.save_interval == 0:         # train.py:121-123
+                os.makedirs(os.path.join(checkpoint_dir, "models"), exist_ok=True)
+                agent.save_snapshot(snapshot_path(checkpoint_dir, episode))
+            rank_state = dict(pool=pool.state_dict(), actor=actor.state_dict() if actor is not None else None,
+                              envs=[e.get_state() if hasattr(e, "get_state") else None for e in envs],
+                              obs=list(obs), done=list(done), history=history,
+                              cpu_rng=torch.get_rng_state(), cuda_rng=torch.cuda.get_rng_state(device))
+            checkpoint.save(checkpoint_dir, episode + 1, rank, learner, ckpt_cfg, rank_state)
     return learner, history
+
+
+def _restore(path, rank, cfg, learner, pool, actor, envs, obs, done, device, log):
+    """Load checkpoint `path` into this rank's learner, pool, actor, environments, per-worker `obs` / `done` (updated in
+    place) and RNG states. Returns (episodes completed, history). An environment without get_state / set_state (e.g.
+    CARLA's) is left freshly reset: training continues, but not on the same trajectory."""
+    shared, mine = checkpoint.load(path, rank, cfg, log)
+    learner.load_state_dict(dict(shared["learner"], rng_states=mine["rng_states"]))
+    checkpoint.check_restored(learner, shared)
+    pool.load_state_dict(mine["pool"])
+    if actor is not None:
+        actor.load_state_dict(mine["actor"])
+    for w, (env, st) in enumerate(zip(envs, mine["envs"])):
+        if st is not None and hasattr(env, "set_state"):
+            env.set_state(st)
+            obs[w], done[w] = mine["obs"][w], mine["done"][w]
+        elif actor is not None:
+            actor.reset(w)
+    torch.set_rng_state(mine["cpu_rng"])
+    torch.cuda.set_rng_state(mine["cuda_rng"], device)
+    return mine["episodes"], list(mine["history"])
 
 
 def _diagnostics_line(episode, d):
@@ -146,7 +203,9 @@ def main():
     if cfg.env_cfg.num_processes % world:
         raise SystemExit(f"env_cfg.num_processes={cfg.env_cfg.num_processes} is not divisible by WORLD_SIZE={world}")
     workers = cfg.env_cfg.num_processes // world
-    train(rank, cfg.train_cfg, cfg.agent_cfg, cfg.env_cfg, cfg.rollout_cfg, danet_state, workers=workers)
+    # CADRE_CHECKPOINT_DIR: snapshots + training checkpoints; CADRE_RESUME: "latest" or an ep_<n> directory
+    train(rank, cfg.train_cfg, cfg.agent_cfg, cfg.env_cfg, cfg.rollout_cfg, danet_state, workers=workers,
+          checkpoint_dir=os.environ.get("CADRE_CHECKPOINT_DIR") or None, resume=os.environ.get("CADRE_RESUME") or None)
 
 
 if __name__ == "__main__":
