@@ -69,39 +69,53 @@ class BatchedActor:
         return (np.array_equal(tick["rgb"][-2], last[0]) and np.array_equal(tick["route_fig"][-2], last[1])
                 and np.array_equal(tick["measurements"][-2], last[2]))
 
-    def encode(self, ticks):
-        """ticks: list of E tick_data dicts. Updates and returns the [E, 8, 530] feature windows."""
-        assert len(ticks) == self.E
-        full = [e for e in range(self.E) if not self._slid_by_one(e, ticks[e])]
+    def _env_list(self, ticks, envs):
+        """The environments `ticks` belongs to: all E in order when `envs` is None, else the listed distinct ids."""
+        if envs is None:
+            assert len(ticks) == self.E
+            return list(range(self.E))
+        envs = [int(e) for e in envs]
+        if len(ticks) != len(envs):
+            raise ValueError(f"{len(ticks)} ticks for {len(envs)} environments")
+        if len(set(envs)) != len(envs) or any(e < 0 or e >= self.E for e in envs):
+            raise ValueError(f"envs must be distinct ids in [0, {self.E}) (got {envs})")
+        return envs
+
+    def encode(self, ticks, envs=None):
+        """ticks: list of E tick_data dicts, or, with `envs` (distinct environment ids), one per listed environment:
+        only those windows are updated, the others stay as they are. Returns the [E, 8, 530] feature windows."""
+        envs = self._env_list(ticks, envs)
+        full = [i for i, e in enumerate(envs) if not self._slid_by_one(e, ticks[i])]
         enc = self.agent.vae_model
         dev = self.agent.vae_device
-        if len(full) < self.E:   # newest frame of every environment whose window slid by one
-            inc = [e for e in range(self.E) if e not in set(full)] if full else list(range(self.E))
+        if len(full) < len(envs):   # newest frame of every environment whose window slid by one
+            inc = [i for i in range(len(envs)) if i not in set(full)] if full else list(range(len(envs)))
             n = len(inc)
             rgb_np, route_np, meas_np = self._rgb_h.numpy(), self._route_h.numpy(), self._meas_h.numpy()
-            for i, e in enumerate(inc):
-                np.copyto(rgb_np[i], ticks[e]["rgb"][-1])
-                np.copyto(route_np[i], ticks[e]["route_fig"][-1])
-                meas_np[i] = ticks[e]["measurements"][-1]
+            for j, i in enumerate(inc):
+                np.copyto(rgb_np[j], ticks[i]["rgb"][-1])
+                np.copyto(route_np[j], ticks[i]["route_fig"][-1])
+                meas_np[j] = ticks[i]["measurements"][-1]
             new = enc.forward_u8(self._rgb_h[:n].to(dev, non_blocking=True), self._route_h[:n].to(dev, non_blocking=True),
                                  self._meas_h[:n].to(dev, non_blocking=True)).to(self.device)
-            if n == self.E:
+            inc_envs = [envs[i] for i in inc]
+            if inc_envs == list(range(self.E)):
                 self.feats[:, :-1] = self.feats[:, 1:].clone()
                 self.feats[:, -1] = new
             else:
-                ids = torch.as_tensor(inc, device=self.device)
+                ids = torch.as_tensor(inc_envs, device=self.device)
                 self.feats[ids, :-1] = self.feats[ids, 1:].clone()
                 self.feats[ids, -1] = new
             self.frames_encoded += n
-        for e in full:   # first tick after a reset (or a window that did not slide): all eight frames
-            t = ticks[e]
-            self.feats[e] = enc.forward_u8(
+        for i in full:   # first tick after a reset (or a window that did not slide): all eight frames
+            t = ticks[i]
+            self.feats[envs[i]] = enc.forward_u8(
                 torch.from_numpy(np.ascontiguousarray(t["rgb"])).to(dev),
                 torch.from_numpy(np.ascontiguousarray(t["route_fig"])).to(dev),
                 torch.from_numpy(np.ascontiguousarray(t["measurements"], dtype=np.float64)).to(dev)).to(self.device)
             self.frames_encoded += self.S
-        for e in range(self.E):
-            t = ticks[e]
+        for i, e in enumerate(envs):
+            t = ticks[i]
             self._last[e] = (np.array(t["rgb"][-1], copy=True), np.array(t["route_fig"][-1], copy=True),
                              np.array(t["measurements"][-1], copy=True))
         return self.feats
@@ -145,8 +159,8 @@ class BatchedActor:
             log_probs.append(logits.gather(1, a))
         return feats, torch.cat(actions, 1), torch.cat(log_probs, 1), out[:, :, 0].t().contiguous()
 
-    def _upload_commands(self, ticks):
-        for e, t in enumerate(ticks):
+    def _upload_commands(self, ticks, envs=None):
+        for e, t in zip(range(self.E) if envs is None else envs, ticks):
             self._cmd_h[e, 0] = int(t["command"])
         cmd = self._cmd_h.to(self.device, non_blocking=True)
         for st in self._st:

@@ -616,7 +616,7 @@ __global__ void __launch_bounds__(256) act_write_kernel(const float* __restrict_
   if (threadIdx.x < 2) {
     const int h = threadIdx.x, A = h == 0 ? 33 : 3;
     const float* row = row_out + (static_cast<long long>(h) * E_env + e) * ROW_OUT;
-    const float u = philox_uniform(philox_word(philox_words(seed, tick, env_ids[e]), h));
+    const float u = philox_uniform(philox_word(philox_words(seed, tick, env_ids[e], 0u), h));
     const int a = categorical_draw(row + 3, A, u);
     const long long at = (2LL * e + h) * T1 + slot;
     pool.action[at] = a;
@@ -641,6 +641,59 @@ __global__ void __launch_bounds__(256) act_write_kernel(const float* __restrict_
       pool.hn[o0 + k] = vh, pool.hn[o1 + k] = vh;
       pool.cn[o0 + k] = vc, pool.cn[o1 + k] = vc;
     }
+  }
+}
+
+// Ensemble tail (cadre_ensemble_control, cadre_ppo_ensemble_act): one warp per environment e. Lane k (and k + 32)
+// picks both heads' actions of snapshot k from row_out[k][h][e] (the sampler keyed with snapshot index k, or the first
+// maximum of the log-probs in greedy mode); lane 0 then averages the snapshots' controls in float64, summed in snapshot
+// order and divided by K, as numpy's mean(0) in CadreAgent.avg_action (agent.py:83-95) does.
+constexpr int ENSEMBLE_MAX_K = 64;
+constexpr int ENSEMBLE_WARPS = 4;
+__device__ __forceinline__ int first_argmax(const float* lp, int A) {   // torch.argmax: the first maximum, NaN wins
+  int best = 0;
+  float bv = lp[0];
+  for (int j = 1; j < A; ++j) {
+    const float v = lp[j];
+    if (bv == bv && (v > bv || v != v)) bv = v, best = j;
+  }
+  return best;
+}
+
+__global__ void __launch_bounds__(ENSEMBLE_WARPS * 32) ensemble_control_kernel(
+    const float* __restrict__ row_out, int K, int E_env, unsigned long long seed, unsigned long long tick,
+    const int* __restrict__ env_ids, int greedy, const double* __restrict__ steer_table,
+    const double* __restrict__ throttle_table, double* __restrict__ controls_out, long long* __restrict__ actions_out) {
+  pdl_trigger();
+  pdl_wait();
+  __shared__ unsigned char act[ENSEMBLE_WARPS][ENSEMBLE_MAX_K][2];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int e = blockIdx.x * ENSEMBLE_WARPS + warp;
+  if (e >= E_env) return;
+  const unsigned env_id = static_cast<unsigned>(env_ids[e]);
+  for (int k = lane; k < K; k += 32) {
+    const uint4 x = greedy ? make_uint4(0u, 0u, 0u, 0u) : philox_words(seed, tick, static_cast<int>(env_id), k);
+    for (int h = 0; h < 2; ++h) {
+      const int A = h == 0 ? 33 : 3;
+      const float* lp = row_out + ((static_cast<long long>(k) * 2 + h) * E_env + e) * ROW_OUT + 3;
+      const int a = greedy ? first_argmax(lp, A) : categorical_draw(lp, A, philox_uniform(philox_word(x, h)));
+      act[warp][k][h] = static_cast<unsigned char>(a);
+      actions_out[(static_cast<long long>(k) * E_env + e) * 2 + h] = a;
+    }
+  }
+  __syncwarp();
+  if (lane == 0) {
+    double steer = 0.0, throttle = 0.0, brake = 0.0;
+    for (int k = 0; k < K; ++k) {
+      const int as = act[warp][k][0], at = act[warp][k][1];
+      steer += steer_table[as];
+      throttle += throttle_table[2 * at];
+      brake += throttle_table[2 * at + 1];
+    }
+    const double n = static_cast<double>(K);
+    steer /= n, throttle /= n, brake /= n;
+    if (K > 1 && brake < 0.5) brake = 0.0;   // agent.py:92-94: several agents release a brake below one half
+    controls_out[3 * e] = steer, controls_out[3 * e + 1] = throttle, controls_out[3 * e + 2] = brake;
   }
 }
 
@@ -1293,6 +1346,77 @@ int cadre_ppo_act(void* handle, const cadre_storage_ref* storages_host, const in
                   reinterpret_cast<long long*>(actions_out));
   CADRE_CUDA_CHECK(cudaGetLastError());
   P->launches = n + 2;
+  CADRE_API_END
+}
+
+}  // extern "C"
+
+namespace cadre {
+static void check_ensemble_args(const float* row_out, int K, int greedy, const int32_t* env_ids,
+                                const double* steer_table, const double* throttle_table, const double* controls_out,
+                                const int64_t* actions_out) {
+  CADRE_REQUIRE(K >= 1 && K <= ENSEMBLE_MAX_K, "ensemble: K must lie in [1, 64]");
+  CADRE_REQUIRE(greedy == 0 || greedy == 1, "ensemble: greedy must be 0 or 1");
+  CADRE_REQUIRE(row_out && env_ids && steer_table && throttle_table && controls_out && actions_out,
+                "ensemble pointers");
+}
+
+static void launch_ensemble_control(const float* row_out, int K, int E_env, uint64_t seed, uint64_t tick,
+                                    const int32_t* env_ids, int greedy, const double* steer_table,
+                                    const double* throttle_table, double* controls_out, int64_t* actions_out,
+                                    cudaStream_t s) {
+  launch_k(ensemble_control_kernel, dim3((E_env + ENSEMBLE_WARPS - 1) / ENSEMBLE_WARPS), dim3(ENSEMBLE_WARPS * 32), 0,
+           s, row_out, K, E_env, static_cast<unsigned long long>(seed), static_cast<unsigned long long>(tick), env_ids,
+           greedy, steer_table, throttle_table, controls_out, reinterpret_cast<long long*>(actions_out));
+  CADRE_CUDA_CHECK(cudaGetLastError());
+}
+}  // namespace cadre
+
+extern "C" {
+
+int cadre_ensemble_control(const float* row_out, int K, int E, uint64_t seed, uint64_t tick, const int32_t* env_ids,
+                           int greedy, const double* steer_table, const double* throttle_table, double* controls_out,
+                           int64_t* actions_out, void* stream) {
+  CADRE_API_BEGIN
+  cadre::check_ensemble_args(row_out, K, greedy, env_ids, steer_table, throttle_table, controls_out, actions_out);
+  CADRE_REQUIRE(E >= 1, "ensemble: E must be at least 1");
+  cadre::launch_ensemble_control(row_out, K, E, seed, tick, env_ids, greedy, steer_table, throttle_table, controls_out,
+                                 actions_out, static_cast<cudaStream_t>(stream));
+  CADRE_API_END
+}
+
+int cadre_ppo_ensemble_act(void* handle, const cadre_storage_ref* storages_host, const int32_t* indices_host,
+                           const float* const* params_host, int K, float* row_out, uint64_t seed, uint64_t tick,
+                           const int32_t* env_ids, int greedy, const double* steer_table, const double* throttle_table,
+                           double* controls_out, int64_t* actions_out, void* stream) {
+  CADRE_API_BEGIN
+  cadre::check_ensemble_args(row_out, K, greedy, env_ids, steer_table, throttle_table, controls_out, actions_out);
+  CADRE_REQUIRE(storages_host && indices_host && params_host, "ppo_ensemble_act pointers");
+  for (int k = 0; k < K; ++k) CADRE_REQUIRE(params_host[k] != nullptr, "ppo_ensemble_act: params_host[k] is NULL");
+  PpoPlan* P = static_cast<PpoPlan*>(handle);
+  CADRE_REQUIRE(P != nullptr, "ppo_ensemble_act: ppo handle is NULL");
+  const int E_env = P->cfg.mini_batch;
+  CADRE_REQUIRE(P->cfg.workers == 1, "ppo_ensemble_act needs an engine with workers = 1, mini_batch = E");
+  for (int h = 0; h < 2; ++h)
+    for (int i = 0; i < E_env; ++i)
+      CADRE_REQUIRE(indices_host[h * E_env + i] == i, "ppo_ensemble_act: indices must be 0..E-1 for both heads");
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  // One upload of the index table for all K forwards: K identical slices, each forward's prep_kernel advances to the
+  // next, so the forwards need no host copy (and no wait on the pinned staging buffer) between snapshots.
+  std::vector<int32_t> tab(static_cast<size_t>(K) * 2 * E_env);
+  for (int k = 0; k < K; ++k) std::copy(indices_host, indices_host + 2 * E_env, tab.begin() + static_cast<size_t>(k) * 2 * E_env);
+  cadre::ppo_stage(P, storages_host, tab.data(), K, P->host_step, s);
+  int n = 0;
+  for (int k = 0; k < K; ++k) {
+    float* rows = row_out + static_cast<size_t>(k) * 2 * E_env * cadre::ROW_OUT;
+    n = cadre::ppo_forward(P, nullptr, nullptr, params_host[k], s);
+    cadre::launch_k(cadre::head_eval_kernel, dim3((2 * P->R + 7) / 8), dim3(256), 0, s, P->Y2, params_host[k],
+                    P->row_slot, P->row_expert, P->sc.action, P->R, P->cap, rows);
+  }
+  CADRE_CUDA_CHECK(cudaGetLastError());
+  cadre::launch_ensemble_control(row_out, K, E_env, seed, tick, env_ids, greedy, steer_table, throttle_table,
+                                 controls_out, actions_out, s);
+  P->launches = K * (n + 1) + 1;
   CADRE_API_END
 }
 

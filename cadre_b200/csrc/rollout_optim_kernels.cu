@@ -17,7 +17,7 @@ __global__ void __launch_bounds__(128) categorical_sample_kernel(const float* __
   pdl_wait();
   const int r = blockIdx.x * blockDim.x + threadIdx.x;
   if (r >= rows) return;
-  const float u = philox_uniform(philox_word(philox_words(seed, tick, env_ids[r]), word));
+  const float u = philox_uniform(philox_word(philox_words(seed, tick, env_ids[r], 0u), word));
   const float* lp = logp + r * ld;
   const int a = categorical_draw(lp, A, u);
   action_out[r] = a;

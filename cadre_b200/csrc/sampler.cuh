@@ -3,7 +3,9 @@
 //
 // A draw is a pure function of (seed, env id, tick, head, log-probs); the library keeps no RNG state, so an
 // environment draws the same actions whichever batch, actor or rank it is stepped in:
-//   x = Philox4x32-10(counter = (tick lo, tick hi, env id, 0), key = (seed lo, seed hi)), word 0 = steer, 1 = throttle;
+//   x = Philox4x32-10(counter = (tick lo, tick hi, env id, k), key = (seed lo, seed hi)), word 0 = steer, 1 = throttle;
+//   k = 0 on the rollout path; an ensemble (cadre_ppo_ensemble_act) keys snapshot k's draws with its index k, so its
+//   snapshot 0 draws exactly what the rollout path would draw for the same (seed, env id, tick);
 //   u = (x >> 8) * 2^-24 (24 bits, exact in fp32, u in [0, 1));
 //   p_j = expf(lp_j), c_j = p_0 + ... + p_j summed in index order, j < A (columns >= A are never read);
 //   a = min{ j : c_j > u * c_{A-1} }, or, if rounding leaves none, max{ j : p_j > 0 } (0 if every p_j is 0).
@@ -13,9 +15,10 @@
 
 namespace cadre {
 
-__device__ __forceinline__ uint4 philox_words(unsigned long long seed, unsigned long long tick, int env_id) {
+__device__ __forceinline__ uint4 philox_words(unsigned long long seed, unsigned long long tick, int env_id,
+                                              unsigned k) {
   const uint4 ctr = make_uint4(static_cast<unsigned>(tick), static_cast<unsigned>(tick >> 32),
-                               static_cast<unsigned>(env_id), 0u);
+                               static_cast<unsigned>(env_id), k);
   const uint2 key = make_uint2(static_cast<unsigned>(seed), static_cast<unsigned>(seed >> 32));
   return curand_Philox4x32_10(ctr, key);
 }

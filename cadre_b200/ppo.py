@@ -147,6 +147,22 @@ class PpoEngine:
                 _lib.ptr(hn), _lib.ptr(cn), _lib.ptr(actions), _lib.stream_ptr(self.device)))
         return actions
 
+    def ensemble_act(self, storages, advantages, indices, params_list, row_out, seed, tick, env_ids, greedy, steer_table,
+                     throttle_table, controls, actions):
+        """cadre_ppo_ensemble_act (workers = 1, mini_batch = E): `evaluate` with each of the K flat parameter tensors of
+        `params_list` into row_out [K, 2, E, 36], then one kernel that picks every snapshot's actions (sampler keyed by
+        seed / tick / env_ids / snapshot index, or the first argmax if `greedy`) into actions int64 [K, E, 2] and
+        averages their controls into controls fp64 [E, 3] (steer_table fp64 [33], throttle_table fp64 [6])."""
+        idx = self._marshal(storages, advantages, indices)
+        K = len(params_list)
+        ptrs = (ctypes.c_void_p * max(K, 1))(*[p.data_ptr() for p in params_list])
+        with torch.cuda.device(self.device):
+            _lib.check(self._lib.cadre_ppo_ensemble_act(
+                self._h, self._refs, idx.ctypes.data_as(ctypes.c_void_p), ptrs, int(K), _lib.ptr(row_out),
+                ctypes.c_uint64(seed), ctypes.c_uint64(tick), _lib.ptr(env_ids), int(greedy), _lib.ptr(steer_table),
+                _lib.ptr(throttle_table), _lib.ptr(controls), _lib.ptr(actions), _lib.stream_ptr(self.device)))
+        return controls, actions
+
     def bootstrap(self, storages, advantages, indices, params, row_out, done_mask, next_value):
         """cadre_ppo_bootstrap (mini_batch = 1): next_value [W, 2] = the value of each worker's row, 0 where bit w of
         done_mask is set; no host synchronisation."""
@@ -274,6 +290,29 @@ def categorical_sample(logp, A, seed, tick, env_ids, word, u_out=None):
             _lib.ptr(logp), int(ld), int(rows), int(A), ctypes.c_uint64(seed), ctypes.c_uint64(tick), _lib.ptr(env_ids),
             int(word), _lib.ptr(action), _lib.ptr(lp), _lib.ptr(u_out), _lib.stream_ptr(logp.device)))
     return action, lp
+
+
+def ensemble_control(row_out, seed, tick, env_ids, steer_table, throttle_table, greedy=False):
+    """cadre_ensemble_control (include/cadre_b200.h): rows fp32 [K, 2, E, 36] in `evaluate`'s format, env_ids int32
+    [E], steer_table fp64 [33], throttle_table fp64 [6]. Returns (controls fp64 [E, 3], actions int64 [K, E, 2])."""
+    _check_tensor(row_out, torch.float32, "row_out")
+    _check_tensor(env_ids, torch.int32, "env_ids")
+    _check_tensor(steer_table, torch.float64, "steer_table")
+    _check_tensor(throttle_table, torch.float64, "throttle_table")
+    if row_out.dim() != 4 or row_out.shape[1] != 2 or row_out.shape[3] != ROW_OUT or env_ids.numel() != row_out.shape[2]:
+        raise _lib.CadreError(f"ensemble_control: row_out must be [K, 2, E, {ROW_OUT}] with E = len(env_ids) "
+                              f"(got {tuple(row_out.shape)}, {env_ids.numel()} env ids)")
+    if steer_table.numel() != 33 or throttle_table.numel() != 6:
+        raise _lib.CadreError("ensemble_control: steer_table needs 33 entries and throttle_table 3 x 2")
+    K, E = row_out.shape[0], row_out.shape[2]
+    controls = torch.empty(E, 3, dtype=torch.float64, device=row_out.device)
+    actions = torch.empty(K, E, 2, dtype=torch.int64, device=row_out.device)
+    with torch.cuda.device(row_out.device):
+        _lib.check(_lib.lib().cadre_ensemble_control(
+            _lib.ptr(row_out), int(K), int(E), ctypes.c_uint64(seed), ctypes.c_uint64(tick), _lib.ptr(env_ids),
+            int(greedy), _lib.ptr(steer_table), _lib.ptr(throttle_table), _lib.ptr(controls), _lib.ptr(actions),
+            _lib.stream_ptr(row_out.device)))
+    return controls, actions
 
 
 def gae(rewards, values, masks, next_value, returns, adv, gamma=0.99, tau=0.95, normalize=True):

@@ -282,7 +282,8 @@ int cadre_ppo_early_stop(void* handle, int32_t* state_host, float* kl_host, int 
  * Counter-based categorical sampler (cadre_b200/csrc/sampler.cuh). A draw is a pure function of
  * (seed, env id, tick, word, log-probs); the library holds no RNG state:
  *   x = Philox4x32-10(counter = (tick & 0xffffffff, tick >> 32, env_id, 0), key = (seed & 0xffffffff, seed >> 32)),
- *       output word `word` (the act step uses word 0 for the steer head, 1 for the throttle head);
+ *       output word `word` (the act step uses word 0 for the steer head, 1 for the throttle head); counter word 3 is
+ *       0 here and the snapshot index k in cadre_ensemble_control;
  *   u = (x >> 8) * 2^-24, exact in fp32;
  *   p_j = expf(lp_j) for j < A (columns >= A are never read), c_j = inclusive prefix sum in index order;
  *   a = min{ j : c_j > u * c_{A-1} }, or max{ j : p_j > 0 } if rounding leaves none; so p_j == 0 is never drawn.
@@ -333,6 +334,33 @@ int cadre_rollout_env_results(const cadre_rollout_pool* pool, int slot, const fl
  * [workers][2] = value of worker w's head h, exactly 0 where bit w of done_mask is set. No host synchronisation. */
 int cadre_ppo_bootstrap(void* handle, const cadre_storage_ref* storages_host, const int32_t* indices_host,
                         const float* params, float* row_out, uint64_t done_mask, float* next_value, void* stream);
+
+/* ------------------------------------------------------------------------------------------------------
+ * Ensemble evaluation (eval.py:53-63): K policy snapshots act on the same E environments and their controls are
+ * averaged (CadreAgent.avg_action, agent.py:83-95).
+ *
+ * cadre_ensemble_control: row_out fp32 [K][2][E][36] in cadre_ppo_evaluate's row format (snapshot k's rows at
+ * row_out + k * 2 * E * 36). For snapshot k, environment e and head h (A = 33 / 3):
+ *   greedy = 0: a = the sampler above with counter (tick lo, tick hi, env_ids[e], k), output word h; snapshot 0 thus
+ *               draws what cadre_ppo_act draws for the same (seed, env id, tick);
+ *   greedy = 1: a = the first index of the largest log-prob among j < A (torch.argmax's rule).
+ * actions_out int64 [K][E][2] = the actions; controls_out fp64 [E][3] = (steer, throttle, brake) averaged over the K
+ * snapshots: steer_table fp64 [33] (STEER_CONTROL), throttle_table fp64 [3][2] ((throttle, brake) = THROTTLE_CONTROL),
+ * the three sums taken in float64 in snapshot order and divided by K, then, if K > 1 and the mean brake is below 0.5,
+ * brake = 0: bit for bit numpy's mean(0) of avg_action. 1 <= K <= 64, E >= 1, greedy in {0, 1}; one launch. */
+int cadre_ensemble_control(const float* row_out, int K, int E, uint64_t seed, uint64_t tick, const int32_t* env_ids,
+                           int greedy, const double* steer_table, const double* throttle_table, double* controls_out,
+                           int64_t* actions_out, void* stream);
+/* One ensemble tick on an engine with workers = 1, mini_batch = E (storages_host / indices_host as for cadre_ppo_act:
+ * the [E][8][530] windows and commands, indices 0..E-1 for both heads): for each snapshot k, the forward plan and
+ * head_eval_kernel with parameters params_host[k] (K device pointers) into row_out[k] (bit-identical to
+ * cadre_ppo_evaluate with those parameters), then cadre_ensemble_control's kernel once. The index table is uploaded
+ * once for all K forwards. cadre_ppo_launches = K * (forward launches + 1) + 1 (the forward's own count is the one
+ * cadre_ppo_evaluate reports, minus its head_eval_kernel). */
+int cadre_ppo_ensemble_act(void* handle, const cadre_storage_ref* storages_host, const int32_t* indices_host,
+                           const float* const* params_host, int K, float* row_out, uint64_t seed, uint64_t tick,
+                           const int32_t* env_ids, int greedy, const double* steer_table, const double* throttle_table,
+                           double* controls_out, int64_t* actions_out, void* stream);
 
 /* ------------------------------------------------------------------------------------------------------
  * Gradient exchange across the ranks of one NVSwitch domain, in place: grads <- sum over ranks, every rank receives
