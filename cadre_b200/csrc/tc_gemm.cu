@@ -163,13 +163,18 @@ static void fill_epilogue(TcGemmParams& p, const GemmArgs& a) {
 }
 
 void launch_gemm(const GemmArgs& a, cudaStream_t stream) {
-  CADRE_REQUIRE(a.M > 0 && a.N > 0 && a.K >= 0 && a.batch > 0, "gemm dims");
+  CADRE_REQUIRE(a.M > 0 && a.N > 0 && a.batch > 0, "gemm dims");
+  CADRE_REQUIRE(a.K > 0, "gemm K must be positive (an empty contraction has no tensor map)");
   CADRE_REQUIRE(a.A && a.B && a.out, "gemm pointers");
+  // the fp32 epilogue reads the ReLU-backward mask as float4 rows (tc_gemm.cuh fast path)
+  CADRE_REQUIRE(!a.mask || !a.out_f32 ||
+                    (reinterpret_cast<uintptr_t>(a.mask) % 16 == 0 && a.ldm % 4 == 0 && a.mask_bs % 4 == 0),
+                "gemm fp32 mask must be 16-byte aligned with ldm and mask_bs multiples of 4");
   CADRE_REQUIRE(a.epi == EPI_LINEAR, "the LSTM-cell epilogue moved into the persistent recurrence kernels (lstm_seq.cuh)");
   const int es = a.kind ? 4 : 2;
   const int bk = 128 / es;
   int bn = a.block_n ? a.block_n : (a.N <= 64 ? 64 : 128);
-  if (a.K > 0 && a.kind == 0 && !a.a_mn && !a.b_mn && a.batch == 1 && !a.out_f32 && a.epi == 0 && !a.mask &&
+  if (a.kind == 0 && !a.a_mn && !a.b_mn && a.batch == 1 && !a.out_f32 && a.epi == 0 && !a.mask &&
       !a.batch_rows && a.alpha == 1.f && a.N % 8 == 0) {
     PersistParams q;
     memset(&q, 0, sizeof(q));

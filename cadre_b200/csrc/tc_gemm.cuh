@@ -116,7 +116,7 @@ __global__ void __launch_bounds__(64 + 128 * EW) tc_gemm_kernel(const __grid_con
     if (p.rows_is_k) {
       num_kb = (cnt + BK - 1) / BK;  // operands are zero padded up to the next multiple of 128 rows
     } else {
-      m_valid = cnt;
+      m_valid = min(cnt, p.M);          // a count above M must not open rows past the output
       if (m_tile * 128 >= cnt) return;  // uniform for the whole CTA, before any barrier
     }
   }

@@ -80,6 +80,39 @@ def test_allreduce_entry_points_validate_their_arguments():
         SwitchAllReduce(1024, "cuda:0")
 
 
+def test_gemm_rejects_an_empty_contraction_and_a_misaligned_fp32_mask():
+    """cadre_gemm refuses, before it builds a tensor map or launches anything: K = 0, and an fp32-output ReLU-backward
+    mask that the epilogue could not read as float4 rows (base not 16-byte aligned, ldm or mask_bs not a multiple of
+    4). Every call also asks for the retired LSTM-cell epilogue (epi = 1), which launch_gemm rejects right after these
+    checks: no call here reaches a tensor map or a launch, with or without a device, and legal masks stop there."""
+    from cadre_b200 import _lib
+    lib = _lib.lib()
+
+    def call(**kw):
+        a = _lib.GemmArgs()
+        a.kind, a.batch, a.M, a.N, a.K, a.alpha, a.out_f32, a.epi = 1, 2, 256, 128, 128, 1.0, 1, 1
+        a.A, a.B, a.out = 0x10000, 0x20000, 0x30000          # never dereferenced
+        a.lda, a.ldb, a.ldc, a.a_bs, a.b_bs, a.out_bs = 128, 128, 128, 256 * 128, 128 * 128, 256 * 128
+        for k, v in kw.items():
+            setattr(a, k, v)
+        rc = lib.cadre_gemm(ctypes.byref(a), None)
+        return rc, lib.cadre_last_error().decode()
+
+    rc, msg = call(K=0)
+    assert rc != 0 and "gemm K must be positive" in msg, msg
+    bad_masks = (dict(mask=0x40004, ldm=128, mask_bs=256 * 128),   # 4-byte aligned base
+                 dict(mask=0x40000, ldm=130, mask_bs=256 * 130),   # ldm not a multiple of 4
+                 dict(mask=0x40000, ldm=128, mask_bs=256 * 128 + 2))
+    for kw in bad_masks:
+        rc, msg = call(**kw)
+        assert rc != 0 and "fp32 mask must be 16-byte aligned" in msg, (kw, msg)
+    # legal masks pass: an aligned fp32 one, and any 16-bit mask (the epilogue reads those per element)
+    for kw in (dict(mask=0x40000, ldm=128, mask_bs=256 * 128),
+               dict(kind=0, out_f32=0, mask=0x40002, ldm=129, mask_bs=3)):
+        rc, msg = call(**kw)
+        assert rc != 0 and "LSTM-cell epilogue" in msg, (kw, msg)
+
+
 def test_product_package_does_not_import_oracle():
     pkg = os.path.join(ROOT, "cadre_b200")
     for dirpath, _, files in os.walk(pkg):

@@ -1,5 +1,6 @@
-"""GPU probe for the tcgen05 tile kernel: prints one line per case (never asserts) so a single gpurun call
-shows every failing descriptor / layout combination at once. Not part of the test-suite."""
+"""GPU probe for the convolution, stem and flat kernels built on the tcgen05 tile kernel: prints one line per case
+(never asserts), so one run shows every failing layout combination at once, plus a few throughput probes. Not part of
+the test-suite: the GEMM instantiations are tested element by element in tests/test_ppo_gemm_gpu.py."""
 import ctypes
 import os
 import sys
@@ -26,83 +27,6 @@ def report(name, got, ref, tol):
     print(f"{'FAIL' if bad else 'ok  '} {name}: max_abs_err={err:.3e} ref_max={scale:.3e} rel={err/scale:.3e}",
           flush=True)
     return not bad
-
-
-def run_gemm(kind, a_mn, b_mn, M, N, K, batch=1, out_f32=1, act=0, bias=False, res=False, block_n=0,
-             rows=None, name=""):
-    dt = torch.float32 if kind else ENC16
-    es = 4 if kind else 2
-    al = 16 // es
-
-    def pad(x):
-        return (x + al - 1) // al * al
-    # logical A [batch, M, K], B [batch, N, K]
-    A = torch.randn(batch, M, K, device=dev).to(dt)
-    Bm = torch.randn(batch, N, K, device=dev).to(dt)
-    if a_mn:
-        lda = pad(M)
-        As = torch.zeros(batch, K, lda, device=dev, dtype=dt)
-        As[:, :, :M] = A.transpose(1, 2)
-        a_bs = K * lda
-    else:
-        lda = pad(K)
-        As = torch.zeros(batch, M, lda, device=dev, dtype=dt)
-        As[:, :, :K] = A
-        a_bs = M * lda
-    if b_mn:
-        ldb = pad(N)
-        Bs = torch.zeros(batch, K, ldb, device=dev, dtype=dt)
-        Bs[:, :, :N] = Bm.transpose(1, 2)
-        b_bs = K * ldb
-    else:
-        ldb = pad(K)
-        Bs = torch.zeros(batch, N, ldb, device=dev, dtype=dt)
-        Bs[:, :, :K] = Bm
-        b_bs = N * ldb
-    odt = torch.float32 if out_f32 else ENC16
-    ldc = (N + 7) // 8 * 8
-    out = torch.full((batch, M, ldc), 7.0, device=dev, dtype=odt)
-    bias_t = torch.randn(batch, N, device=dev) if bias else None
-    res_t = torch.randn(batch, M, ldc, device=dev).to(odt) if res else None
-    rows_t = torch.tensor(rows, device=dev, dtype=torch.int32) if rows is not None else None
-    g = _lib.GemmArgs()
-    g.kind, g.a_mn, g.b_mn, g.batch = kind, a_mn, b_mn, batch
-    g.M, g.N, g.K, g.block_n = M, N, K, block_n
-    g.A, g.B = As.data_ptr(), Bs.data_ptr()
-    g.lda, g.a_bs, g.ldb, g.b_bs = lda, a_bs, ldb, b_bs
-    g.out, g.ldc, g.out_bs = out.data_ptr(), ldc, M * ldc
-    g.out_f32, g.act = out_f32, act
-    if bias:
-        g.bias, g.bias_bs = bias_t.data_ptr(), N
-    if res:
-        g.res, g.ldr, g.res_bs = res_t.data_ptr(), ldc, M * ldc
-    if rows is not None:
-        g.batch_rows = rows_t.data_ptr()
-    g.alpha = 1.0
-    rc = L.cadre_gemm(ctypes.byref(g), _lib.stream_ptr())
-    if rc != 0:
-        print(f"FAIL {name}: rc={rc} {L.cadre_last_error().decode()}", flush=True)
-        return False
-    torch.cuda.synchronize()
-    Af, Bf = A.float(), Bm.float()
-    ref = torch.bmm(Af.double(), Bf.double().transpose(1, 2)).float()
-    if bias:
-        ref = ref + bias_t[:, None, :]
-    if res:
-        ref = ref + res_t[:, :, :N].float()
-    if act == 1:
-        ref = ref.relu()
-    if act == 2:
-        ref = F.leaky_relu(ref, 0.01)
-    got = out[:, :, :N].float()
-    if rows is not None:
-        for b, r in enumerate(rows):
-            ref[b, r:] = 0
-            # rows beyond the last processed tile keep the fill value; only compare processed tiles
-            last = min(M, (r + 127) // 128 * 128)
-            got[b, last:] = 0
-    tol = 2e-3 if kind else (1e-2 if not out_f32 else 1e-4)
-    return report(name, got, ref, tol)
 
 
 def run_conv(B, H, W, Cin, Cout, k, stride, pad, act=1, res=False, name=""):
@@ -217,8 +141,6 @@ def timed(fn, iters=20):
 def main():
     group = sys.argv[1] if len(sys.argv) > 1 else "all"
     print(L.cadre_version().decode(), torch.cuda.get_device_name(0), group, flush=True)
-    if group in ("all", "gemm"):
-        gemm_cases()
     if group in ("all", "conv"):
         conv_cases()
     if group in ("all", "stem"):
@@ -232,22 +154,6 @@ def main():
         run_conv_inpad(3, 36, 64, 64, 128, 1, 2, 0, name="conv1x1 s2 from padded input")
     if group in ("all", "perf"):
         perf_cases()
-
-
-def gemm_cases():
-    run_gemm(0, 0, 0, 128, 128, 64, name="bf16 KK 128x128x64")
-    run_gemm(0, 0, 0, 256, 128, 256, name="bf16 KK 256x128x256")
-    run_gemm(0, 0, 0, 300, 200, 104, name="bf16 KK tails 300x200x104")
-    run_gemm(0, 0, 0, 256, 64, 512, name="bf16 KK N=64")
-    run_gemm(0, 0, 0, 256, 256, 512, out_f32=0, act=1, bias=True, res=True, name="bf16 KK bf16-out bias+res+relu")
-    run_gemm(0, 0, 1, 256, 256, 256, name="bf16 K/MN 256^3")
-    run_gemm(0, 1, 1, 256, 256, 256, name="bf16 MN/MN 256^3")
-    run_gemm(1, 0, 0, 128, 128, 32, name="tf32 KK 128x128x32")
-    run_gemm(1, 0, 0, 200, 2120, 530, bias=True, name="tf32 KK 200x2120x530")
-    run_gemm(1, 0, 1, 200, 530, 2120, name="tf32 K/MN dgrad 200x530x2120")
-    run_gemm(1, 1, 1, 2120, 530, 200, name="tf32 MN/MN wgrad 2120x530x200")
-    run_gemm(1, 0, 0, 300, 256, 530, batch=4, rows=[300, 130, 0, 77], name="tf32 KK batched rows")
-    run_gemm(1, 0, 0, 128, 64, 128, name="tf32 KK N=64")
 
 
 def conv_cases():
